@@ -6,6 +6,7 @@ inference on one B200 (weights: oracle.synth random-init, spectral norm converge
 oracle.synth.synthetic_slices).  One "step" = one generator forward over one batch of 16 slices.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--precision fp32|bf16] [--impl reference] [--no-extras]
+                  [--dump-outputs DIR]
 
 * value      : slices/s with inputs resident in HBM; every step is timed with its own CUDA-event pair
                on the launching stream and L2 is flushed (256 MiB write) between steps.
@@ -23,6 +24,9 @@ oracle.synth.synthetic_slices).  One "step" = one generator forward over one bat
                (pix2pix training step, global batch 16 sharded over the ranks, NCCL gradient all-reduce) and
                config 5 (volumes sharded over the ranks, no collective).
 * --impl reference : the reference's CPU implementation on all host threads, same config / metric.
+* --dump-outputs DIR : after the run, the seven outputs Generator.forward returned in the last timed step, as
+               DIR/<name>.npy (float32, full size).  Weights and inputs are seeded, so the files of two builds compare
+               output for output; with --impl reference they are the reference forward's outputs for rank 0's batch.
 Multi-GPU (torchrun): weak scaling, every rank runs its own batch-16 stream of slices, no collective
 on the data path; barrier + synchronize around the timed region, max over ranks.
 """
@@ -40,6 +44,7 @@ sys.path.insert(0, ROOT)
 BATCH = 16
 FLOP_PER_SLICE = 17.54e9          # SURVEY.md §8(d): 14.187 (47 convs) + 1.208 + 2.147 (attention) GFLOP
 METRIC = "slices/sec two-stage gen fwd (256x256)"
+OUTPUT_NAMES = ("coarse_seg", "fine_seg", "x_stage1", "x_stage2", "flow", "pred1_h", "pred2_h")   # Generator.forward's tuple
 WORKLOAD = f"batch-{BATCH} 256x256 two-stage generator inference (BASELINE.json configs[1])"
 
 
@@ -137,9 +142,9 @@ def _cpu_forward_rate(steps, warmup, batch=BATCH):
             fwd(x, mask, cam, ratio)
         t0 = time.perf_counter()
         for _ in range(steps):
-            fwd(x, mask, cam, ratio)
+            out = fwd(x, mask, cam, ratio)
         dt = time.perf_counter() - t0
-    return batch * steps / dt, dt / steps * 1e3, torch.get_num_threads(), kind
+    return batch * steps / dt, dt / steps * 1e3, torch.get_num_threads(), kind, out
 
 
 def run_reference(args, rank, world):
@@ -147,7 +152,7 @@ def run_reference(args, rank, world):
         return
     # the CPU arm needs ~0.4 s per batch-16 step (each step = the full batch): the requested step count is kept up to 200 (80 s)
     steps = max(1, min(args.steps, 200))
-    rate, ms, threads, kind = _cpu_forward_rate(steps, args.warmup)
+    rate, ms, threads, kind, out = _cpu_forward_rate(steps, args.warmup)
     what = "the unmodified reference modules (oracle/_ref)" if kind == "reference" else "oracle port of the reference"
     sample = f"{steps} steps x batch {BATCH} (each step = one full batch-{BATCH} forward), {what}"
     line = {
@@ -161,6 +166,8 @@ def run_reference(args, rank, world):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, host_outputs(out))
 
 
 # ------------------------------------------------------------------------------------------------ extras
@@ -398,13 +405,15 @@ def run_ours(args, rank, world, local_rank):
         flush.fill_(1)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        step()
+        out = step()
         e1.record(stream)
         evs.append((e0, e1))
     barrier()
     wall = time.perf_counter() - wall0
     launches = _lib.launch_count() - launches0
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
+    # host copies of the last timed step's outputs, taken before anything else runs on the generator; written at the end
+    dumped = host_outputs(out) if args.dump_outputs and rank == 0 else None
 
     # ---------------- end to end through the public uint8 HOST interface (hv_pipeline_*), 4 slots in flight
     rng = np.random.Generator(np.random.PCG64(1000 + rank))
@@ -546,13 +555,28 @@ def run_ours(args, rank, world, local_rank):
             "extra": extra,
         }
         if world == 1 and not args.no_cpu_baseline:
-            rate, ms, threads, kind = _cpu_forward_rate(10, 1)
+            rate, ms, threads, kind, _ = _cpu_forward_rate(10, 1)
             what = "the unmodified reference modules (oracle/_ref)" if kind == "reference" else "oracle port of the reference forward"
             line["cpu_baseline"] = {"value": rate, "unit": "slices/s", "cores": threads, "kind": kind,
                                     "sample": f"10 steps x batch {BATCH} of the same workload ({ms:.0f} ms/step), {what}"}
         print(json.dumps(line), flush=True)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
+
+
+def host_outputs(out):
+    """Generator.forward's 7-tuple as named float32 host arrays."""
+    return {name: t.float().cpu().numpy() for name, t in zip(OUTPUT_NAMES, out)}
+
+
+def dump_outputs(directory, arrays):
+    """One float32 .npy per output of Generator.forward, full size (about 28 MB for batch 16)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def main():
@@ -565,7 +589,12 @@ def main():
                     help="bf16 = tcgen05 tensor-core mode (headline); fp32 = SIMT parity mode")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the `extra` sub-records (configs 3/4/5, fp32 mode, torch baselines)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0's batch; with --impl reference, the reference "
+                         "forward's) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
