@@ -912,6 +912,8 @@ void tc_set_trace(long long* dev_buf) { g_trace = dev_buf; }
 static long long* g_timeline = nullptr;
 static int g_timeline_count = 0;
 void tc_set_timeline(long long* dev_buf) { g_timeline = dev_buf; g_timeline_count = 0; }
+bool tc_pdl_enabled() { return g_pdl; }
+long long* tc_timeline_next() { return g_timeline ? g_timeline + 4 * (g_timeline_count++) : nullptr; }
 
 template <int N_PAD, int ACT, int FIXED = 0, bool DIAG = true>
 static int tc_launch_na(const TcConv& c, cudaStream_t st) {

@@ -186,6 +186,39 @@ bool tc_trunk_eligible(const TcConv& c);
 size_t tc_trunk_counter_ints(int max_images);
 int tc_trunk_launch(const TcConv* const* convs, int count, int n_images, int* counters, cudaStream_t st);
 
+// fused thin tail of a generator stage (tail_tc.cu): a 16 -> 8 x-phase 3x3 ELU conv and the dual heads that read its output (plus
+// chunk 1 of the heads' own source buffer) in one persistent launch; the 8-channel intermediate stays in shared memory
+struct TcTailParams {
+  CUtensorMap maps[4];   // conv input: views 1-4, shifted views; heads' second chunk: views 1-4, shifted views
+  const void* w_mid;     // packed weights / padded bias of the two per-layer instances (TcConv::w_packed, bias_pad)
+  const void* w_head;
+  const float* bias_mid;
+  const float* bias_head;
+  int n, h, w_img;
+  int rows_per_unit, strips, units;   // work unit = (image pair, strip of rows_per_unit output rows)
+  float* head0;
+  float* head1;
+  TcAux aux0;            // bf16 copy of head 0 (coarse stage: x_stage1 for the fine heads), or ptr == null
+  TcBuf kx;              // head 1 kx-packed (5 taps, channels 0-4 of chunk kx_chunk; coarse stage: the fine conv1 input), or ptr == null
+  int kx_chunk;
+  long long* timeline;
+};
+struct TcTail {
+  TcTailParams p;
+  int grid = 0;
+};
+// mid: the 16 -> 8 conv (x-phase source, chunked output), heads: the dual-head instance reading mid's output buffer; the weights are
+// read from the instances' packed buffers at launch time
+int tc_tail_setup(TcTail& t, const TcConv& mid, const TcConv& heads, int n_images);
+void tc_tail_set_batch(TcTail& t, int n_images);
+void tc_tail_set_outputs(TcTail& t, float* head0, float* head1);
+// also write head 1 as tc_pack_kx(k = 5, dil = 1) would into chunk `chunk` of dst (null: off)
+int tc_tail_set_kxpack(TcTail& t, const TcBuf* dst, int chunk);
+int tc_tail_launch(const TcTail& t, cudaStream_t st);
+// launch helpers shared with conv_tc.cu: programmatic dependent launch on (HV_NO_PDL unset), next slot of the timeline hook (or null)
+bool tc_pdl_enabled();
+long long* tc_timeline_next();
+
 // fp32 NCHW <-> chunked bf16 converters (channel c of the source lands in chunk c/8, lane c%8)
 int tc_pack_nchw(const float* src, int src_channels, int mode /*hv_src_mode*/, const TcBuf& dst, int dst_channel0,
                  cudaStream_t st);

@@ -283,7 +283,17 @@ struct TcPlan {
   __nv_bfloat16* blob = nullptr;
   int* trunk_ctr = nullptr;            // [kNumLayers][tc_trunk_counter_ints(max_batch)]: queue / completion counters of the chain starting at a layer
   size_t trunk_ctr_stride = 0;
+  // the 16 -> 8 conv + dual heads of each stage as ONE launch (tail_tc.cu): conv16 -> conv17 | conv18, allconv16 -> allconv17 | allconv18
+  TcTail tail[2];
+  bool tail_fused_last = false;        // the last forward ran the fused tails: B_C16 / chunk 0 of B_A16CAT were not written
 };
+
+// HV_NO_TAIL_FUSE=1: the per-layer launches for the thin tails (A/B runs, parity tests); read once per process.  The fused kernel reads
+// x-phase buffers, so HV_NO_XP implies the per-layer launches too.
+static bool tail_fuse_enabled() {
+  static const bool on = !(getenv("HV_NO_TAIL_FUSE") && atoi(getenv("HV_NO_TAIL_FUSE")) != 0) && !getenv("HV_NO_XP");
+  return on;
+}
 
 // A run of consecutive 64 -> 64 trunk layers, either one launch per layer (programmatic dependent launches) or ONE dataflow launch
 // (trunk_tc.cu).  Measured on B200 (profiles/r2_trunk_dataflow.md): at batch 16 a layer is only 3.7 tile rounds per SM, less than the
@@ -378,6 +388,14 @@ static int tc_plan_create(hv_generator* g) {
       t->out_buf[s.layer] = s.out; t->out_up2[s.layer] = s.up2;
     }
   }
+  if (tail_fuse_enabled()) {
+    int rc = tc_tail_setup(t->tail[0], t->conv[C16], t->conv[C17], n);
+    if (!rc) rc = tc_tail_setup(t->tail[1], t->conv[A16], t->conv[A17], n);
+    // the coarse heads also write the kx-packed coarse mask of the fine network's input (chunk 2 of B_IN_F, see kFineInputMap): the
+    // packing launch between the coarse tail and fine conv1 drops out of the critical path
+    if (!rc) rc = tc_tail_set_kxpack(t->tail[0], &t->buf[B_IN_F], 2);
+    if (rc) return rc;
+  }
   return HV_OK;
 }
 
@@ -444,12 +462,23 @@ static int forward_bf16(hv_generator* g, const float* x, const float* mask, cons
   RC(fork_aux(2));   // the height head reads conv10_atrous (:90-93); nothing of the trunk overwrites it
   RC(tc_gap_fc_sigmoid(view(B_C10), g->fc_w[0], g->fc_b[0], pred1_h, t->gap_partial, t->gap_ticket, ax));
   if (use_aux) HV_CUDA(cudaStreamWaitEvent(st, g->ev_aux[1], 0));
-  for (int l : {C20, C13, C14, C19, C15, C16}) RC(run(l, st));
-  t->conv[C17].p.head0 = x_stage1; t->conv[C17].p.head1 = coarse_seg;
-  RC(run(C17, st));
+  const bool fuse_tail = tail_fuse_enabled();
+  // the heads of a stage and the conv before them: one fused launch (tail_tc.cu), or conv16 + the dual-head instance
+  auto tail = [&](int which, int conv, int heads, float* head0, float* head1) -> int {
+    if (fuse_tail) {
+      tc_tail_set_batch(t->tail[which], n);
+      tc_tail_set_outputs(t->tail[which], head0, head1);
+      return tc_tail_launch(t->tail[which], st);
+    }
+    RC(run(conv, st));
+    t->conv[heads].p.head0 = head0; t->conv[heads].p.head1 = head1;
+    return run(heads, st);
+  };
+  for (int l : {C20, C13, C14, C19, C15}) RC(run(l, st));
+  RC(tail(0, C16, C17, x_stage1, coarse_seg));
   // ---- fine network: xnow = [xin, coarse_seg, mask, ratio]; conv1 | pmconv1 as one 32-filter conv, then the
   // attention branch forks onto the side stream
-  {
+  if (!fuse_tail) {   // the fused coarse tail writes chunk 2 itself (chunk 3 is zero padding, never written)
     const TcPlaneSrc in_f1[1] = {{coarse_seg, HV_SRC_DIRECT}};   // chunks 2-3: the only part packed on the critical path
     RC(tc_pack_kx(in_f1, 1, 5, 1, view(B_IN_F).chunk_view(2, 2), st));
   }
@@ -470,9 +499,9 @@ static int forward_bf16(hv_generator* g, const float* x, const float* mask, cons
   RC(fork_aux(4));
   RC(tc_gap_fc_sigmoid(view(B_A11), g->fc_w[1], g->fc_b[1], pred2_h, t->gap_partial + g->max_batch * 8, t->gap_ticket + g->max_batch, ax));
   RC(chain({A12, A19}, st));
-  for (int l : {A13, A14, A15, A16}) RC(run(l, st));
-  t->conv[A17].p.head0 = x_stage2; t->conv[A17].p.head1 = fine_seg;
-  RC(run(A17, st));
+  for (int l : {A13, A14, A15}) RC(run(l, st));
+  RC(tail(1, A16, A17, x_stage2, fine_seg));
+  t->tail_fused_last = fuse_tail;
   RC(join_aux(5));
   g->last_heads[0] = x_stage1; g->last_heads[1] = coarse_seg; g->last_heads[2] = x_stage2; g->last_heads[3] = fine_seg;
   g->last_n = n;
@@ -657,6 +686,13 @@ long long hv_generator_read_tap(hv_generator* g, int idx, float* out, hv_stream_
       HV_CHECK_ARG(b >= 0, "generator_read_tap: layer %d has no tap in bf16 mode", idx);
       TcBuf v = g->tc->buf[b];
       v.n = g->last_n;
+      if (g->tc->tail_fused_last && (idx == C16 || idx == A16)) {
+        // the fused tail kept this layer's output in shared memory: recompute it with the per-layer instance from its input
+        // (B_C15 / B_A15), which the forward leaves intact
+        tc_set_batch(g->tc->conv[idx], g->last_n);
+        int rc = tc_conv_launch(g->tc->conv[idx], as_stream(stream));
+        if (rc) return rc;
+      }
       const int ch = idx == A16 ? 8 : kLayers[idx].cout;
       // layers whose output is stored nearest-x2-upsampled (conv12, conv14, allconv19, allconv14): read the native grid back
       int rc = tc_unpack_nchw(v, 0, ch, out, as_stream(stream), g->tc->out_up2[idx] ? 2 : 1);

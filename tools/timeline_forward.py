@@ -13,7 +13,10 @@ x, mask, cam, ratio = (t.cuda() for t in synth.synthetic_slices(n, seed=1))
 L = _lib.lib()
 L.hv_debug_conv_timeline.argtypes = [ctypes.c_void_p]
 order = ("C1 C2 C3 C4 C5 C6 C7 C8 C9 C10 C11 C12 C20 C13 C14 C19 C15 C16 C17 F1 PM2 PM3 PM4 PM5 PM6 PM9 PM10 "
-         "F2 F3 F4 F5 F6 F7 F8 F9 F10 A11 A12 A19 A13 A14 A15 A16 A17").split()
+         "F2 F3 F4 F5 F6 F7 F8 F9 F10 A11 A12 A19 A13 A14 A15 A16 A17")
+if int(os.environ.get("HV_NO_TAIL_FUSE") or 0) == 0:   # conv16 + heads of each stage run as one fused launch (CTAIL / ATAIL)
+    order = order.replace("C16 C17", "CTAIL").replace("A16 A17", "ATAIL")
+order = order.split()
 with torch.no_grad():
     for _ in range(3):
         g(x, mask, cam, ratio)
