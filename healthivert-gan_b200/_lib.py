@@ -84,8 +84,6 @@ SIGNATURES = {
     "hv_bucket_copy": (c_int, [c_void_p, c_int, c_longlong, c_void_p, c_float, c_int, c_void_p]),
     "hv_debug_conv_trace": (c_int, [c_void_p]),
     "hv_debug_conv_timeline": (c_int, [c_void_p]),
-    "hv_debug_trunk_trace": (c_int, [c_void_p, c_int]),
-    "hv_debug_backward_paths": (c_int, [c_int]),
     "hv_act_bwd_bias": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "hv_sn_prepare_multi": (c_int, [c_void_p, c_int, c_int, c_void_p]),
     "hv_sn_bwd_multi": (c_int, [c_void_p, c_int, c_void_p]),

@@ -157,7 +157,7 @@ __host__ __device__ constexpr int tc_ctas_per_sm(int n_pad) { return n_pad <= 32
 //   FIXED = kind << 12 | rows << 8 | taps << 4 | k-steps;  kind 1: plain segments of one shape, 2: space-to-depth (k-steps),
 //   3: x-phase (rows, k-steps), 4: two sources, segment 0 = (3 rows, 3 taps, k-steps), segment 1 = kx-packed plane (3, 1, 1)
 __host__ __device__ constexpr int tc_shape_code(int kind, int rows, int taps, int ksteps) { return kind << 12 | rows << 8 | taps << 4 | ksteps; }
-// DIAG: the diagnostics (per-role clock trace, launch timeline stamps, HV_TC_DEBUG ablation bits) are compiled in only for the
+// DIAG: the diagnostics (per-role clock trace, launch timeline stamps) are compiled in only for the
 // instances that the host picks while a diagnostic is active: in the production instances they cost 2.4 % of the forward (the
 // single-thread loops pay for every extra instruction).
 template <int N_PAD, int ACT, int FIXED = 0, bool DIAG = true>
@@ -242,7 +242,6 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
     int slot = 0, ntr = 0;
     uint32_t phase = 0;
     long long* tr = (DIAG && p.trace && blockIdx.x == 0) ? p.trace : nullptr;
-    const int debug = DIAG ? p.debug : 0;
     const unsigned long long tiles_magic = p.tiles_magic;
     const int tiles_per_image = p.tiles_per_image, tile_adv = p.tile_adv, q_first = p.q_first, total_tiles = p.total_tiles;
     const uint32_t slots_base = smem_u32(s_slots);
@@ -251,8 +250,6 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
     const uint32_t slot_bytes = p.slot_bytes;
     int rel2 = p.segs[0].rel_start2, c1 = p.segs[0].c1;   // single-segment layers keep the load recipe in registers
     uint32_t tx = p.segs[0].tx_bytes;
-    int cpl = p.segs[0].cpl, nload = p.segs[0].nload;
-    uint32_t load_bytes = p.segs[0].load_bytes;
     bool map1 = false;
     const int rounds = (total_tiles + TPR - 1) / TPR;
     for (int round = blockIdx.x; round < rounds; round += gridDim.x) {
@@ -266,19 +263,17 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
       for (int s = 0; s < nseg; ++s) {
         if (nseg > 1) {
           rel2 = p.segs[s].rel_start2; c1 = p.segs[s].c1; tx = p.segs[s].tx_bytes; map1 = p.segs[s].map != 0;
-          cpl = p.segs[s].cpl; nload = p.segs[s].nload; load_bytes = p.segs[s].load_bytes;
         }
         mbar_wait(bar_empty + 8u * slot, phase ^ 1u);
         if (leader) {
           const uint32_t fb = bar_full + 8u * slot, dst = slots_base + (uint32_t)slot * slot_stride;
-          mbar_expect_tx(fb, (debug & 2) ? 0u : tx * TPR);
-          for (int i = 0; i < ((debug & 2) ? 0 : nload); ++i) {
-            if (map5d) tma_load_5d(dst + (uint32_t)i * load_bytes, &p.maps[0], fb, c_tile + rel2, c1, 0, i * cpl, img);   // {positions, rows, 4 sub-planes / phases, chunks, image}
-            else tma_load_4d(dst + (uint32_t)i * load_bytes, map1 ? &p.maps[1] : &p.maps[0], fb, c_tile + rel2, c1, i * cpl, img);
-            if (PAIR) {
-              if (map5d) tma_load_5d(dst + slot_bytes + (uint32_t)i * load_bytes, &p.maps[0], fb, c_tile_b + rel2, c1, 0, i * cpl, img_b);
-              else tma_load_4d(dst + slot_bytes + (uint32_t)i * load_bytes, map1 ? &p.maps[1] : &p.maps[0], fb, c_tile_b + rel2, c1, i * cpl, img_b);
-            }
+          mbar_expect_tx(fb, tx * TPR);
+          // one operation per band: the box spans all chunks of the segment
+          if (map5d) tma_load_5d(dst, &p.maps[0], fb, c_tile + rel2, c1, 0, 0, img);   // {positions, rows, 4 sub-planes / phases, chunks, image}
+          else tma_load_4d(dst, map1 ? &p.maps[1] : &p.maps[0], fb, c_tile + rel2, c1, 0, img);
+          if (PAIR) {
+            if (map5d) tma_load_5d(dst + slot_bytes, &p.maps[0], fb, c_tile_b + rel2, c1, 0, 0, img_b);
+            else tma_load_4d(dst + slot_bytes, map1 ? &p.maps[1] : &p.maps[0], fb, c_tile_b + rel2, c1, 0, img_b);
           }
           trace_ev(tr, ntr, 1);
         }
@@ -288,7 +283,6 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
   } else if (warp == W_MMA) {
     // ===================================================================== MMA issuer (warp-uniform, one lane issues)
     const bool leader = elect_one();
-    const bool mma_on = leader && !(DIAG && (p.debug & 1));
     // instruction descriptor: D=f32, A=B=bf16, both K-major, N = N_PAD, M = 128
     constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N_PAD >> 3) << 17) | ((128u >> 4) << 24);
     // smem descriptor = hi word (SBO = 128 B, version 1) : lo word (start >> 4 | LBO >> 4 << 16); offsets add into lo.
@@ -339,15 +333,15 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
           for (int u = 0; u < TPR; ++u) {   // the tiles of the round: band u of the slot -> accumulator u of the stage
             const uint32_t dt = d_tmem + (uint32_t)(u * N_PAD), au = (uint32_t)u * slot_units;
             if (FK == 1) {
-              issue_segment<N_PAD, FR ? FR : 1, FT ? FT : 1, FS ? FS : 1>(mma_on, dt, a_row + au, b_row, a_step, b_step, b_row_step, idesc, accumulate);
+              issue_segment<N_PAD, FR ? FR : 1, FT ? FT : 1, FS ? FS : 1>(leader, dt, a_row + au, b_row, a_step, b_step, b_row_step, idesc, accumulate);
             } else if (FK == 2) {
-              issue_s2d<N_PAD, FS ? FS : 1>(mma_on, dt, a_slot + au + ((8u * TC_TILE_M) << 16), b_row, b_step, idesc);
+              issue_s2d<N_PAD, FS ? FS : 1>(leader, dt, a_slot + au + ((8u * TC_TILE_M) << 16), b_row, b_step, idesc);
             } else if (FK == 3) {
-              issue_xp4<N_PAD, FR ? FR : 1, FS ? FS : 1>(mma_on, dt, a_slot + au + ((4u * (uint32_t)(FR ? FR : 1) * TC_TILE_M) << 16), b_row, b_step, idesc,
+              issue_xp4<N_PAD, FR ? FR : 1, FS ? FS : 1>(leader, dt, a_slot + au + ((4u * (uint32_t)(FR ? FR : 1) * TC_TILE_M) << 16), b_row, b_step, idesc,
                                                        accumulate);
             } else {
-              if (s == 0) issue_segment<N_PAD, 3, 3, FS ? FS : 1>(mma_on, dt, a_row + au, b_row, a_step, b_step, b_row_step, idesc, accumulate);
-              else issue_segment<N_PAD, 3, 1, 1>(mma_on, dt, a_row + au, b_row, a_step, b_step, b_row_step, idesc, accumulate);
+              if (s == 0) issue_segment<N_PAD, 3, 3, FS ? FS : 1>(leader, dt, a_row + au, b_row, a_step, b_step, b_row_step, idesc, accumulate);
+              else issue_segment<N_PAD, 3, 1, 1>(leader, dt, a_row + au, b_row, a_step, b_step, b_row_step, idesc, accumulate);
             }
           }
           accumulate = 1;
@@ -356,9 +350,9 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
         }
         if (s2d) {
           const uint32_t a_s2d = a_slot + ((8u * TC_TILE_M) << 16);
-          if (ksteps == 1) issue_s2d<N_PAD, 1>(mma_on, d_tmem, a_s2d, b_row, b_step, idesc);
-          else if (ksteps == 2) issue_s2d<N_PAD, 2>(mma_on, d_tmem, a_s2d, b_row, b_step, idesc);
-          else issue_s2d<N_PAD, 4>(mma_on, d_tmem, a_s2d, b_row, b_step, idesc);
+          if (ksteps == 1) issue_s2d<N_PAD, 1>(leader, d_tmem, a_s2d, b_row, b_step, idesc);
+          else if (ksteps == 2) issue_s2d<N_PAD, 2>(leader, d_tmem, a_s2d, b_row, b_step, idesc);
+          else issue_s2d<N_PAD, 4>(leader, d_tmem, a_s2d, b_row, b_step, idesc);
           accumulate = 1;
           if (leader) { umma_commit(cur_empty); trace_ev(tr, ntr, 13); }
           continue;
@@ -367,10 +361,10 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
           const uint32_t a_xp = a_slot + ((4u * (uint32_t)nrows * TC_TILE_M) << 16);
           const int shape_xp = (nrows << 4) | ksteps;
           switch (shape_xp) {
-            case (3 << 4) | 1: issue_xp4<N_PAD, 3, 1>(mma_on, d_tmem, a_xp, b_row, b_step, idesc, accumulate); break;
-            case (3 << 4) | 2: issue_xp4<N_PAD, 3, 2>(mma_on, d_tmem, a_xp, b_row, b_step, idesc, accumulate); break;
-            case (1 << 4) | 1: issue_xp4<N_PAD, 1, 1>(mma_on, d_tmem, a_xp, b_row, b_step, idesc, accumulate); break;
-            default: issue_xp4<N_PAD, 1, 2>(mma_on, d_tmem, a_xp, b_row, b_step, idesc, accumulate); break;
+            case (3 << 4) | 1: issue_xp4<N_PAD, 3, 1>(leader, d_tmem, a_xp, b_row, b_step, idesc, accumulate); break;
+            case (3 << 4) | 2: issue_xp4<N_PAD, 3, 2>(leader, d_tmem, a_xp, b_row, b_step, idesc, accumulate); break;
+            case (1 << 4) | 1: issue_xp4<N_PAD, 1, 1>(leader, d_tmem, a_xp, b_row, b_step, idesc, accumulate); break;
+            default: issue_xp4<N_PAD, 1, 2>(leader, d_tmem, a_xp, b_row, b_step, idesc, accumulate); break;
           }
           accumulate = 1;
           if (leader) { umma_commit(cur_empty); trace_ev(tr, ntr, 13); }
@@ -379,14 +373,14 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
         const int shape = (nrows << 8) | (ntaps << 4) | ksteps;
 #define HV_SEG(R, T, K)                                                                                                   \
   case ((R) << 8) | ((T) << 4) | (K):                                                                                     \
-    issue_segment<N_PAD, R, T, K>(mma_on, d_tmem, a_row, b_row, a_step, b_step, b_row_step, idesc, accumulate);           \
+    issue_segment<N_PAD, R, T, K>(leader, d_tmem, a_row, b_row, a_step, b_step, b_row_step, idesc, accumulate);           \
     break;
         switch (shape) {
           HV_SEG(3, 3, 1) HV_SEG(3, 3, 2) HV_SEG(3, 3, 4) HV_SEG(5, 5, 1) HV_SEG(5, 5, 2)
           HV_SEG(1, 3, 1) HV_SEG(1, 3, 2) HV_SEG(1, 3, 4) HV_SEG(1, 2, 1) HV_SEG(1, 2, 2) HV_SEG(1, 1, 1) HV_SEG(1, 1, 2)
           HV_SEG(5, 1, 1) HV_SEG(5, 1, 2) HV_SEG(1, 5, 1) HV_SEG(3, 1, 1) HV_SEG(1, 1, 4)
           default:
-            issue_segment_generic<N_PAD>(mma_on, d_tmem, a_row, b_row, a_step, b_step, b_row_step, idesc, accumulate, nrows, ntaps, ksteps);
+            issue_segment_generic<N_PAD>(leader, d_tmem, a_row, b_row, a_step, b_step, b_row_step, idesc, accumulate, nrows, ntaps, ksteps);
         }
 #undef HV_SEG
         accumulate = 1;
@@ -421,7 +415,7 @@ __global__ void __launch_bounds__(tc_threads(N_PAD), tc_ctas_per_sm(N_PAD)) conv
       const int yy = qrow - p.in_border;
       const int xx = q - qrow * p.in_pitch - p.in_border;
       // rows >= tile_adv read past the band (their taps shift beyond position 127): garbage, skipped
-      const bool valid = m < p.tile_adv && yy >= 0 && yy < p.h_out && xx >= 0 && xx < p.w_out && !(DIAG && (p.debug & 4));
+      const bool valid = m < p.tile_adv && yy >= 0 && yy < p.h_out && xx >= 0 && xx < p.w_out;
       trace_ev(tr, ntr, 20);
       mbar_wait(bar_tfull + 8u * acc, acc_phase);
       tc_fence_after();
@@ -544,7 +538,7 @@ static PFN_encodeTiled get_encode() {
 //   stride-1 sources : dims {positions*2, k rows, chunks, n}, dim 1 steps `dil` image rows, so ONE box of `box_rows`
 //                      rows brings the bands of `box_rows` kernel rows (the dims overlap in memory; TMA does not mind)
 //   s2d sources      : dims {sub-plane positions*2, 4 sub-planes, chunks, n}, box_rows = 1
-static int make_map(CUtensorMap* map, const TcBuf& b, int box_chunks, int k, int dil, int box_rows) {
+static int make_map(CUtensorMap* map, const TcBuf& b, int k, int dil, int box_rows) {
   PFN_encodeTiled enc = get_encode();
   if (!enc) { set_error("cuTensorMapEncodeTiled is unavailable (driver entry point lookup failed)"); return HV_ERR_CUDA; }
   const cuuint64_t plane_b = (cuuint64_t)b.plane() * 16, sub_b = (cuuint64_t)b.sub_plane() * 16;
@@ -554,7 +548,7 @@ static int make_map(CUtensorMap* map, const TcBuf& b, int box_chunks, int k, int
     if (!b.s2d && b.xp == 1) {
       cuuint64_t dims[4] = {(cuuint64_t)b.sub_plane() * 2, (cuuint64_t)k, (cuuint64_t)b.chunks, (cuuint64_t)b.n};
       cuuint64_t strides[3] = {(cuuint64_t)dil * b.pitch() * 16, plane_b, plane_b * b.image_chunks()};
-      cuuint32_t box[4] = {2 * TC_TILE_M, (cuuint32_t)box_rows, (cuuint32_t)box_chunks, 1};
+      cuuint32_t box[4] = {2 * TC_TILE_M, (cuuint32_t)box_rows, (cuuint32_t)b.chunks, 1};
       cuuint32_t es[4] = {1, 1, 1, 1};
       r = enc(map, types[attempt], 4, b.ptr, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -562,7 +556,7 @@ static int make_map(CUtensorMap* map, const TcBuf& b, int box_chunks, int k, int
       // x-phase source: {positions*2, k rows, xp phases, chunks, n}; one box = `box_rows` kernel rows of all phases
       cuuint64_t dims[5] = {(cuuint64_t)b.sub_plane() * 2, (cuuint64_t)k, (cuuint64_t)b.xp, (cuuint64_t)b.chunks, (cuuint64_t)b.n};
       cuuint64_t strides[4] = {(cuuint64_t)dil * b.pitch() * 16, sub_b, plane_b, plane_b * b.image_chunks()};
-      cuuint32_t box[5] = {2 * TC_TILE_M, (cuuint32_t)box_rows, (cuuint32_t)b.xp, (cuuint32_t)box_chunks, 1};
+      cuuint32_t box[5] = {2 * TC_TILE_M, (cuuint32_t)box_rows, (cuuint32_t)b.xp, (cuuint32_t)b.chunks, 1};
       cuuint32_t es[5] = {1, 1, 1, 1, 1};
       r = enc(map, types[attempt], 5, b.ptr, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -570,7 +564,7 @@ static int make_map(CUtensorMap* map, const TcBuf& b, int box_chunks, int k, int
       // space-to-depth source: {positions*2, 2 rows (dy = -1, 0), 4 parity sub-planes, chunks, n}: one box = everything a tile needs
       cuuint64_t dims[5] = {(cuuint64_t)b.sub_plane() * 2, 2, 4, (cuuint64_t)b.chunks, (cuuint64_t)b.n};
       cuuint64_t strides[4] = {(cuuint64_t)b.pitch() * 16, sub_b, plane_b, plane_b * b.image_chunks()};
-      cuuint32_t box[5] = {2 * TC_TILE_M, 2, 4, (cuuint32_t)box_chunks, 1};
+      cuuint32_t box[5] = {2 * TC_TILE_M, 2, 4, (cuuint32_t)b.chunks, 1};
       cuuint32_t es[5] = {1, 1, 1, 1, 1};
       r = enc(map, types[attempt], 5, b.ptr, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -633,7 +627,6 @@ int tc_conv_setup(TcConv& c, const TcSource* srcs, int nsrc, int k, int stride, 
   const int pitch = b0.pitch();
   HV_CHECK_ARG((long long)b0.plane() < (1ll << 20), "tc_conv: plane too large for the fast row division");
   p.s2d_in = stride == 2;
-  if (const char* e = getenv("HV_TC_DEBUG")) p.debug = atoi(e);
   p.in_xp = xp; p.cp = cp; p.map5d = (stride == 2 || xp > 1) ? 1 : 0;
   p.ups = ups ? 1 : 0;
   p.w_img = b0.w;
@@ -649,15 +642,13 @@ int tc_conv_setup(TcConv& c, const TcSource* srcs, int nsrc, int k, int stride, 
   // Tile pairs (see PAIR in the kernel) for a thin, long layer that cannot run as two co-resident CTAs (its three band slots do not
   // fit in half the shared memory): at least ~6 rounds per SM and two pair slots beside the weights.  Measured per layer on B200:
   // pairs help exactly there (merged fine conv1|pmconv1: 45.0 -> 40.5 us); where two CTAs per SM are possible they are the better
-  // latency hiding (pairs: conv3 +4 us, heads +8 us), and the x-phase layers lose too (conv16 +3 us).  HV_TC_PAIR=0 switches the
-  // mode off (A/B).
+  // latency hiding (pairs: conv3 +4 us, heads +8 us), and the x-phase layers lose too (conv16 +3 us).
   bool want_pair = false;
   {
-    const char* e = getenv("HV_TC_PAIR");
     const long long est_tiles = ((long long)b0.sub_h() * pitch / (TC_TILE_M - 2) + 1) * n_images;
     const size_t half = (227 * 1024) / 2 - 2048, band = (size_t)TC_TILE_M * max_chunks_of(srcs, nsrc) * 16u * (stride == 2 ? 8 : k * xp);
     const bool two_ctas = tc_ctas_per_sm(c.n_pad) == 2 && fixed + 3 * band <= half;
-    want_pair = allow_pair && !(e && atoi(e) == 0) && c.n_pad <= 32 && xp == 1 && !two_ctas && est_tiles >= 12ll * 148 && fixed + 2 * 2 * band <= budget;
+    want_pair = allow_pair && c.n_pad <= 32 && xp == 1 && !two_ctas && est_tiles >= 12ll * 148 && fixed + 2 * 2 * band <= budget;
   }
   if (!want_pair)
   {  // two co-resident CTAs when the layer is thin and three tile slots still fit in half the shared memory (measured: with
@@ -714,18 +705,6 @@ int tc_conv_setup(TcConv& c, const TcSource* srcs, int nsrc, int k, int stride, 
   }
   p.nseg = seg;
   for (int i = 0; i < seg; ++i) p.segs[i].tx_bytes = (uint32_t)TC_TILE_M * p.segs[i].nchunks * 16u * p.segs[i].nrows * (xp > 1 ? xp : 1);
-  // chunks per TMA operation: 0 = the whole band in one operation.  Measured (HV_TMA_CPL = 1 / 2 / 4): splitting a band into
-  // concurrent operations changes nothing, the ingest rate is set by shared-memory bandwidth shared with the MMA operand reads
-  int cpl_req = 0;
-  if (const char* e = getenv("HV_TMA_CPL")) cpl_req = atoi(e);
-  for (int i = 0; i < seg; ++i) {
-    const int nch = p.segs[i].nchunks;
-    int cpl = (cpl_req <= 0 || cpl_req > nch) ? nch : cpl_req;
-    while (nch % cpl) --cpl;
-    p.segs[i].cpl = cpl;
-    p.segs[i].nload = nch / cpl;
-    p.segs[i].load_bytes = p.segs[i].tx_bytes / (uint32_t)(nch / cpl);
-  }
   p.tile_adv = TC_TILE_M - max_shift;
   const int span = p.h_out * pitch;  // positions from output (0,0) to the end of the last row (incl. side borders)
   p.tiles_per_image = (span + p.tile_adv - 1) / p.tile_adv;
@@ -739,9 +718,7 @@ int tc_conv_setup(TcConv& c, const TcSource* srcs, int nsrc, int k, int stride, 
   p.nslots = nslots;
   c.smem = fixed + (size_t)nslots * slot_stride;
   for (int s = 0; s < nsrc; ++s) {
-    int cpl = srcs[s].buf.chunks;
-    for (int i = 0; i < seg; ++i) if (p.segs[i].map == s) cpl = p.segs[i].cpl;
-    int rc = make_map(&p.maps[s], srcs[s].buf, cpl, k, dil, box_rows);
+    int rc = make_map(&p.maps[s], srcs[s].buf, k, dil, box_rows);
     if (rc) return rc;
   }
   if (nsrc == 1) p.maps[1] = p.maps[0];
@@ -907,12 +884,10 @@ int tc_conv_pack_weights(TcConv& c, const float* wa, const float* ba, int cout_a
 }
 
 static long long* g_trace = nullptr;
-static bool g_pdl = getenv("HV_NO_PDL") == nullptr;
 void tc_set_trace(long long* dev_buf) { g_trace = dev_buf; }
 static long long* g_timeline = nullptr;
 static int g_timeline_count = 0;
 void tc_set_timeline(long long* dev_buf) { g_timeline = dev_buf; g_timeline_count = 0; }
-bool tc_pdl_enabled() { return g_pdl; }
 long long* tc_timeline_next() { return g_timeline ? g_timeline + 4 * (g_timeline_count++) : nullptr; }
 
 template <int N_PAD, int ACT, int FIXED = 0, bool DIAG = true>
@@ -933,7 +908,7 @@ static int tc_launch_na(const TcConv& c, cudaStream_t st) {
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = g_pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   TcParams q = c.p;
   q.trace = g_trace;
   q.timeline = g_timeline ? g_timeline + 4 * (g_timeline_count++) : nullptr;
@@ -958,8 +933,6 @@ static int tc_fixed_code(const TcConv& c) {
 }
 static int tc_issue_code(const TcConv& c) {
   const TcParams& p = c.p;
-  static const bool no_fixed = getenv("HV_TC_NO_FIXED") != nullptr;
-  if (no_fixed) return 0;
   const TcSeg& s0 = p.segs[0];
   const int ks = s0.nchunks >> 1;
   if (p.s2d_in) return p.nseg == 1 ? tc_shape_code(2, 0, 0, ks) : 0;
@@ -1030,8 +1003,8 @@ static int tc_launch_n(const TcConv& c, cudaStream_t st) {
   if (dump) fprintf(stderr, "tc_launch: X(%d, %s, %d << 20 | %d << 16 | tc_shape_code(%d, %d, %d, %d))\n", N_PAD, act == HV_ACT_ELU ? "HV_ACT_ELU" : (act == HV_ACT_RELU ? "HV_ACT_RELU" : "-1"),
                                     fixed >> 20 & 1, fixed >> 16 & 15, (fixed >> 12) & 15, (fixed >> 8) & 15, (fixed >> 4) & 15, fixed & 15);
   if (c.p.pair && !(fixed >> 20 & 1)) { set_error("tc_conv: a paired layer needs a specialised kernel instance"); return HV_ERR_UNSUPPORTED; }
-  // a diagnostic is active (trace / timeline hook set, or ablation bits from HV_TC_DEBUG): the instances that carry the hooks
-  const bool diag = g_trace != nullptr || g_timeline != nullptr || c.p.debug != 0;
+  // a diagnostic is active (trace / timeline hook set): the instances that carry the hooks
+  const bool diag = g_trace != nullptr || g_timeline != nullptr;
 #define HV_TC_TRY(NP, A, F)                                                                                      \
   if (N_PAD == (NP) && act == (A) && fixed == (F))                                                              \
     return diag ? tc_launch_na<NP, A, (N_PAD == (NP) ? (F) : 0), true>(c, st)                                   \

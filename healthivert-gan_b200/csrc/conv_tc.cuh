@@ -76,9 +76,6 @@ struct TcSeg {
   int ntaps;          // taps per row
   uint32_t a0, a_step, b0, b_step, b_row_step;
   uint32_t tx_bytes;  // bytes this load brings
-  int cpl;            // channel chunks per TMA operation: the band is brought by nload = nchunks / cpl operations on one barrier
-  int nload;          // (precomputed on the host: the producer is one thread, an integer division costs it ~100 cycles)
-  uint32_t load_bytes;
 };
 
 enum TcOutMode { TC_OUT_CHUNKED = 0, TC_OUT_CHUNKED_UP2 = 1, TC_OUT_HEADS = 2, TC_OUT_CHUNKED_S2D = 3 };
@@ -120,7 +117,6 @@ struct TcParams {
   int nslots;
   long long* trace;  // debug event trace (device buffer of 12000 int64) or null
   long long* timeline;  // debug: {min CTA entry, max CTA exit} globaltimer ns of this launch, or null
-  int debug;         // ablation bits for bottleneck hunting (env HV_TC_DEBUG): 1 no MMAs, 2 no TMA loads, 4 no output stores
 };
 
 struct TcSource {
@@ -181,11 +177,6 @@ int tc_conv_launch(const TcConv& c, cudaStream_t st);
 void tc_set_trace(long long* dev_buf);  // debug: CTA 0 of every subsequent launch records its event timeline
 void tc_conv_free(TcConv& c);
 
-// dataflow kernel for chains of 64 -> 64 3x3 layers on the 64x64 trunk (trunk_tc.cu): one persistent launch per chain
-bool tc_trunk_eligible(const TcConv& c);
-size_t tc_trunk_counter_ints(int max_images);
-int tc_trunk_launch(const TcConv* const* convs, int count, int n_images, int* counters, cudaStream_t st);
-
 // fused thin tail of a generator stage (tail_tc.cu): a 16 -> 8 x-phase 3x3 ELU conv and the dual heads that read its output (plus
 // chunk 1 of the heads' own source buffer) in one persistent launch; the 8-channel intermediate stays in shared memory
 struct TcTailParams {
@@ -215,8 +206,7 @@ void tc_tail_set_outputs(TcTail& t, float* head0, float* head1);
 // also write head 1 as tc_pack_kx(k = 5, dil = 1) would into chunk `chunk` of dst (null: off)
 int tc_tail_set_kxpack(TcTail& t, const TcBuf* dst, int chunk);
 int tc_tail_launch(const TcTail& t, cudaStream_t st);
-// launch helpers shared with conv_tc.cu: programmatic dependent launch on (HV_NO_PDL unset), next slot of the timeline hook (or null)
-bool tc_pdl_enabled();
+// next slot of the timeline hook (or null), shared with conv_tc.cu
 long long* tc_timeline_next();
 
 // fp32 NCHW <-> chunked bf16 converters (channel c of the source lands in chunk c/8, lane c%8)

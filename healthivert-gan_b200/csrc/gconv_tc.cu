@@ -10,8 +10,6 @@
 // dx is the gradient over the VIRTUAL concatenated input [n, cin, hin, win] of the forward descriptor, exactly like hv_conv2d_dgrad;
 // the host routes channel ranges back to their source tensors.  fp32 SIMT kernels (train_ops.cu) remain the parity path.
 #include <cuda_bf16.h>
-#include <stdio.h>
-#include <stdlib.h>
 #include "hv_common.cuh"
 #include "kernels.h"
 
@@ -329,14 +327,8 @@ struct GpGeom {
   int nrep, rep_shift[5];         // replica j = DY moved right by rep_shift[j] (0 .. 7) positions
 };
 
-// A/B switches (environment HV_DGRAD_GEMM / HV_WGRAD_IM2COL, or hv_debug_backward_paths): bit 0: data gradient through the GEMM +
-// col2im path for every layer, bit 1: weight gradient through the explicit im2col operand for every layer
-static int g_backward_paths = -1;
-
 static bool gp_eligible(const hv_conv_desc* d) {
-  if (g_backward_paths < 0) g_backward_paths = (getenv("HV_DGRAD_GEMM") ? 1 : 0) | (getenv("HV_WGRAD_IM2COL") ? 2 : 0);
-  const bool off = (g_backward_paths & 2) != 0;
-  return !off && (d->win & 7) == 0 && d->stride == 1 && (d->k == 3 || d->k == 5) && d->pad == (d->k - 1) / 2 * d->dil && d->cout <= 128 && d->cin <= 256;
+  return (d->win & 7) == 0 && d->stride == 1 && (d->k == 3 || d->k == 5) && d->pad == (d->k - 1) / 2 * d->dil && d->cout <= 128 && d->cin <= 256;
 }
 
 static void gp_geom(GpGeom& q, const GcGeom& g) {
@@ -492,26 +484,14 @@ int conv2d_wgrad_bf16(const hv_conv_desc* d, const float* dy, float* dw, float* 
     __nv_bfloat16* X = (__nv_bfloat16*)base;
     __nv_bfloat16* DY = (__nv_bfloat16*)(base + gc_al((size_t)g.n * g.cin * q.plane * 2));
     float* part = (float*)((char*)DY + gc_al((size_t)g.n * q.nrep * g.cout * q.plane * 2));
-    static const bool dbg = getenv("HV_GP_DEBUG") != nullptr;
-#define GP_DBG(what)                                                                                                        \
-  if (dbg) {                                                                                                                \
-    cudaError_t e = cudaStreamSynchronize(st);                                                                              \
-    fprintf(stderr, "gp wgrad: %s -> %s (plane %d pitch %d co8 %d tpm %d ntg %d bn %d kb0 %d kblocks %d nkc %d)\n", what,  \
-            cudaGetErrorString(e), q.plane, q.pitch, q.co8, q.tpm, q.ntg, q.bn, q.kb0, q.kblocks, q.nkc);                   \
-  }
     gp_planes_x_kernel<<<gc_blocks((long long)g.n * g.cin * (q.plane >> 3)), 256, 0, st>>>(g, q, X);
     HV_LAUNCH_CHECK();
-    GP_DBG("planes_x");
     gp_planes_dy_kernel<<<gc_blocks((long long)g.n * g.cout * (q.plane >> 3)), 256, 0, st>>>(dy, g, q, DY);
     HV_LAUNCH_CHECK();
-    GP_DBG("planes_dy");
     rc = gemm_tc_taps(DY, X, part, g.n, g.cout, g.cin, q.plane, q.tap_off, q.tap_rep, q.nrep, g.kk, q.tpm, q.co8, q.bn, q.nkc, q.kb0, q.kblocks, st);
     if (rc) return rc;
-    GP_DBG("gemm_tc_taps");
     gp_reduce_dw_kernel<<<(unsigned)((g.cout * g.cin * g.kk + 31) / 32), 256, 0, st>>>(part, dw, g.n * q.nkc, g.cout, g.cin, g.kk, q.tpm, q.ntg, q.co8, q.bn);
     HV_LAUNCH_CHECK();
-    GP_DBG("reduce");
-#undef GP_DBG
     if (db) return channel_sum(dy, db, g.n, g.cout, g.P, st);
     return HV_OK;
   }
@@ -545,9 +525,7 @@ int conv2d_dgrad_bf16(const hv_conv_desc* d, const float* w, const float* dy, fl
     HV_LAUNCH_CHECK();
     return HV_OK;
   }
-  if (g_backward_paths < 0) g_backward_paths = (getenv("HV_DGRAD_GEMM") ? 1 : 0) | (getenv("HV_WGRAD_IM2COL") ? 2 : 0);
-  const bool gemm_dgrad = (g_backward_paths & 1) != 0;   // A/B switch: the GEMM + col2im path for every layer
-  if (!gemm_dgrad && d->stride == 1 && (d->k == 3 || d->k == 5) && d->pad == (d->k - 1) / 2 * d->dil && d->cin <= 64) {
+  if (d->stride == 1 && (d->k == 3 || d->k == 5) && d->pad == (d->k - 1) / 2 * d->dil && d->cin <= 64) {
     // stride-1 'same' convolution (41 of the generator's 47 layers): dx = conv(dy, flipped / transposed filters) on the implicit-GEMM
     // tcgen05 kernel of the forward - no dyT / dcolT operands, no col2im pass.  fp32 accumulation over all taps, ONE rounding to bf16.
     float* wf = reinterpret_cast<float*>(base);
@@ -575,7 +553,6 @@ int conv2d_dgrad_bf16(const hv_conv_desc* d, const float* w, const float* dy, fl
 }  // namespace hv
 
 extern "C" {
-int hv_debug_backward_paths(int bits) { hv::g_backward_paths = bits; return 0; }
 size_t hv_conv2d_wgrad_bf16_workspace_bytes(const hv_conv_desc* d) { return hv::gconv_wgrad_workspace_bytes(d); }
 size_t hv_conv2d_dgrad_bf16_workspace_bytes(const hv_conv_desc* d) { return hv::gconv_dgrad_workspace_bytes(d); }
 int hv_conv2d_wgrad_bf16(const hv_conv_desc* d, const float* dy, float* dw, float* db, void* workspace, hv_stream_t s) {

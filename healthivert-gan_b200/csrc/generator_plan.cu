@@ -281,40 +281,15 @@ struct TcPlan {
   float* gap_partial = nullptr;      // [2][max_batch * 8] shares of the two height heads
   unsigned int* gap_ticket = nullptr;  // [2][max_batch]
   __nv_bfloat16* blob = nullptr;
-  int* trunk_ctr = nullptr;            // [kNumLayers][tc_trunk_counter_ints(max_batch)]: queue / completion counters of the chain starting at a layer
-  size_t trunk_ctr_stride = 0;
   // the 16 -> 8 conv + dual heads of each stage as ONE launch (tail_tc.cu): conv16 -> conv17 | conv18, allconv16 -> allconv17 | allconv18
   TcTail tail[2];
   bool tail_fused_last = false;        // the last forward ran the fused tails: B_C16 / chunk 0 of B_A16CAT were not written
 };
 
-// HV_NO_TAIL_FUSE=1: the per-layer launches for the thin tails (A/B runs, parity tests); read once per process.  The fused kernel reads
-// x-phase buffers, so HV_NO_XP implies the per-layer launches too.
+// HV_NO_TAIL_FUSE=1: the per-layer launches for the thin tails (A/B runs, parity tests); read once per process.
 static bool tail_fuse_enabled() {
-  static const bool on = !(getenv("HV_NO_TAIL_FUSE") && atoi(getenv("HV_NO_TAIL_FUSE")) != 0) && !getenv("HV_NO_XP");
+  static const bool on = !(getenv("HV_NO_TAIL_FUSE") && atoi(getenv("HV_NO_TAIL_FUSE")) != 0);
   return on;
-}
-
-// A run of consecutive 64 -> 64 trunk layers, either one launch per layer (programmatic dependent launches) or ONE dataflow launch
-// (trunk_tc.cu).  Measured on B200 (profiles/r2_trunk_dataflow.md): at batch 16 a layer is only 3.7 tile rounds per SM, less than the
-// dependency hop (TMA + MMA + epilogue + publish ~ 3 rounds): the dataflow kernel needs 17 us per layer against 11 us for separate
-// launches, so it is used from HV_TRUNK_MIN_BATCH images on (default: never; HV_TRUNK=1 forces it, for A/B runs and the parity tests).
-static int run_layers(hv_generator* g, const int* layers, int count, int n, cudaStream_t st) {
-  TcPlan* t = g->tc;
-  static const int force = getenv("HV_TRUNK") ? atoi(getenv("HV_TRUNK")) : 0;
-  static const int min_batch = getenv("HV_TRUNK_MIN_BATCH") ? atoi(getenv("HV_TRUNK_MIN_BATCH")) : (1 << 30);
-  bool ok = (force == 1 || n >= min_batch) && count >= 2 && count <= 8;
-  const TcConv* convs[8];
-  for (int i = 0; i < count; ++i) {
-    tc_conv_set_batch(t->conv[layers[i]], n);
-    if (ok) { convs[i] = &t->conv[layers[i]]; ok = tc_trunk_eligible(*convs[i]) && (i == count - 1 || !t->out_up2[layers[i]]); }
-  }
-  if (ok) return tc_trunk_launch(convs, count, n, t->trunk_ctr + (size_t)layers[0] * t->trunk_ctr_stride, st);
-  for (int i = 0; i < count; ++i) {
-    int rc = tc_conv_launch(t->conv[layers[i]], st);
-    if (rc) return rc;
-  }
-  return HV_OK;
 }
 
 static TcAux make_aux(const TcBuf& b, int channel) {
@@ -327,7 +302,7 @@ static TcAux make_aux(const TcBuf& b, int channel) {
 static void tc_plan_destroy(hv_generator* g) {
   if (!g->tc) return;
   for (int i = 0; i < kNumLayers; ++i) if (g->tc->has[i]) tc_conv_free(g->tc->conv[i]);
-  cudaFree(g->tc->blob); cudaFree(g->tc->ca_ws); cudaFree(g->tc->gap_partial); cudaFree(g->tc->gap_ticket); cudaFree(g->tc->trunk_ctr);
+  cudaFree(g->tc->blob); cudaFree(g->tc->ca_ws); cudaFree(g->tc->gap_partial); cudaFree(g->tc->gap_ticket);
   delete g->tc;
   g->tc = nullptr;
 }
@@ -337,14 +312,13 @@ static int tc_plan_create(hv_generator* g) {
   g->tc = t;
   const int n = g->max_batch;
   size_t total = 0;
-  const bool no_xp = getenv("HV_NO_XP") != nullptr;   // A/B switch: plain layout for the thin 256x256 tail
   for (int i = 0; i < B_COUNT; ++i) {
     TcBuf& b = t->buf[i];
     b.n = n; b.chunks = kBufs[i].channels / 8; b.h = b.w = kBufs[i].extent; b.border = kBufs[i].border;
     // buffers consumed by a stride-2 conv are stored space-to-depth
     b.s2d = (i == B_C1 || i == B_C3 || i == B_F1 || i == B_F3 || i == B_P1 || i == B_P3);
     // inputs of the thin 256x256 tail layers (<= 16 filters: conv15/16/17+18, allconv15/16/17+18) are stored in 4 x-phases
-    b.xp = (!no_xp && (i == B_C19 || i == B_C15 || i == B_C16 || i == B_A15 || i == B_A16CAT)) ? 4 : 1;
+    b.xp = (i == B_C19 || i == B_C15 || i == B_C16 || i == B_A15 || i == B_A16CAT) ? 4 : 1;
     total += (b.bytes() + 255) & ~(size_t)255;
   }
   total += TcBuf::kSlackBytes;
@@ -360,9 +334,6 @@ static int tc_plan_create(hv_generator* g) {
   HV_CUDA(cudaMalloc((void**)&t->gap_partial, sizeof(float) * 2 * n * 8));
   HV_CUDA(cudaMalloc((void**)&t->gap_ticket, sizeof(unsigned int) * 2 * n));
   HV_CUDA(cudaMemset(t->gap_ticket, 0, sizeof(unsigned int) * 2 * n));
-  t->trunk_ctr_stride = tc_trunk_counter_ints(n);
-  HV_CUDA(cudaMalloc((void**)&t->trunk_ctr, sizeof(int) * t->trunk_ctr_stride * kNumLayers));
-  HV_CUDA(cudaMemset(t->trunk_ctr, 0, sizeof(int) * t->trunk_ctr_stride * kNumLayers));
   for (int i = 0; i < kNumLayers; ++i) t->out_buf[i] = -1;
   t->out_buf[PM1] = B_P1;
   for (int i = 0; i < kNumTcLayers; ++i) {
@@ -456,9 +427,7 @@ static int forward_bf16(hv_generator* g, const float* x, const float* mask, cons
     if (use_aux) HV_CUDA(cudaEventRecord(g->ev_aux[1], ax));
   }
   // ---- coarse network
-  auto chain = [&](std::initializer_list<int> ls, cudaStream_t s) -> int { return run_layers(g, ls.begin(), (int)ls.size(), n, s); };
-  for (int l : {C1, C2, C3, C4}) RC(run(l, st));
-  RC(chain({C5, C6, C7, C8, C9, C10, C11, C12}, st));   // the 64x64 trunk of the coarse network: one dataflow launch
+  for (int l : {C1, C2, C3, C4, C5, C6, C7, C8, C9, C10, C11, C12}) RC(run(l, st));
   RC(fork_aux(2));   // the height head reads conv10_atrous (:90-93); nothing of the trunk overwrites it
   RC(tc_gap_fc_sigmoid(view(B_C10), g->fc_w[0], g->fc_b[0], pred1_h, t->gap_partial, t->gap_ticket, ax));
   if (use_aux) HV_CUDA(cudaStreamWaitEvent(st, g->ev_aux[1], 0));
@@ -486,20 +455,17 @@ static int forward_bf16(hv_generator* g, const float* x, const float* mask, cons
   HV_CUDA(cudaEventRecord(g->ev_fork, st));
   HV_CUDA(cudaStreamWaitEvent(g->side, g->ev_fork, 0));
   cudaStream_t sa = g->side;
-  for (int l : {PM2, PM3, PM4}) RC(run(l, sa));
-  RC(chain({PM5, PM6}, sa));
+  for (int l : {PM2, PM3, PM4, PM5, PM6}) RC(run(l, sa));
   RC(ctx_attn_fwd_tc(view(B_P6), mask, view(B_CA), offsets, flow, 10.f, 1, per_sample_mask, t->ca_ws, sa, use_aux ? ax : nullptr,
                      use_aux ? &g->ev_aux[6] : nullptr));
-  RC(chain({PM9, PM10}, sa));
+  for (int l : {PM9, PM10}) RC(run(l, sa));
   HV_CUDA(cudaEventRecord(g->ev_join, sa));
-  for (int l : {F2, F3, F4, F5}) RC(run(l, st));
-  RC(chain({F6, F7, F8, F9, F10}, st));
+  for (int l : {F2, F3, F4, F5, F6, F7, F8, F9, F10}) RC(run(l, st));
   HV_CUDA(cudaStreamWaitEvent(st, g->ev_join, 0));
   RC(run(A11, st));
   RC(fork_aux(4));
   RC(tc_gap_fc_sigmoid(view(B_A11), g->fc_w[1], g->fc_b[1], pred2_h, t->gap_partial + g->max_batch * 8, t->gap_ticket + g->max_batch, ax));
-  RC(chain({A12, A19}, st));
-  for (int l : {A13, A14, A15}) RC(run(l, st));
+  for (int l : {A12, A19, A13, A14, A15}) RC(run(l, st));
   RC(tail(1, A16, A17, x_stage2, fine_seg));
   t->tail_fused_last = fuse_tail;
   RC(join_aux(5));
@@ -653,12 +619,14 @@ int hv_generator_run_chain(hv_generator* g, int first, int count, int n, hv_stre
   HV_CHECK_ARG(g && g->tc, "generator_run_chain: needs a bf16 plan");
   if (!g->prepared) { set_error("generator_run_chain: call hv_generator_prepare first"); return HV_ERR_STATE; }
   HV_CHECK_ARG(n >= 1 && n <= g->max_batch && count >= 1 && first >= 0 && first + count <= kNumLayers, "generator_run_chain: bad range");
-  int layers[kNumLayers];
-  for (int idx = first; idx < first + count; ++idx) {
+  for (int idx = first; idx < first + count; ++idx)
     HV_CHECK_ARG(g->tc->has[idx] && g->tc->out_buf[idx] >= 0, "generator_run_chain: layer %d is not a stand-alone tensor-core conv", idx);
-    layers[idx - first] = idx;
+  for (int idx = first; idx < first + count; ++idx) {
+    tc_set_batch(g->tc->conv[idx], n);
+    int rc = tc_conv_launch(g->tc->conv[idx], as_stream(stream));
+    if (rc) return rc;
   }
-  return run_layers(g, layers, count, n, as_stream(stream));
+  return HV_OK;
 }
 
 long long hv_generator_read_tap(hv_generator* g, int idx, float* out, hv_stream_t stream) {

@@ -455,7 +455,7 @@ int tc_tail_launch(const TcTail& t, cudaStream_t st) {
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = tc_pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   TcTailParams q = t.p;
   q.timeline = tc_timeline_next();
   HV_CUDA(cudaLaunchKernelEx(&cfg, tail_tc_kernel, q));

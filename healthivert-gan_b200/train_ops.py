@@ -427,16 +427,14 @@ class TensorTable:
 
 class FusedAdam:
     """torch.optim.Adam(lr, betas) semantics (pix2pix_model.py:127-130); state keys mirror torch's.  ONE kernel launch per step for
-    all parameters of the optimiser (hv_adam_step_multi); HV_ADAM_PER_TENSOR=1 keeps the one-launch-per-tensor path (A/B)."""
+    all parameters of the optimiser (hv_adam_step_multi); parameters with different step counts take one launch per tensor."""
 
     def __init__(self, params, lr=2e-4, betas=(0.5, 0.999), eps=1e-8):
-        import os
         self.params = [p for p in params]
         self.param_groups = [{"params": self.params, "lr": lr, "initial_lr": lr, "betas": betas, "eps": eps}]
         self.state = {}
         self._table = TensorTable()
         self._step = 0
-        self._per_tensor = os.environ.get("HV_ADAM_PER_TENSOR") == "1"
 
     def zero_grad(self, set_to_none=True):
         for p in self.params:
@@ -452,7 +450,7 @@ class FusedAdam:
             if p not in self.state:
                 self.state[p] = {"step": 0, "exp_avg": torch.zeros_like(p), "exp_avg_sq": torch.zeros_like(p)}
         steps = {self.state[p]["step"] for p in live}
-        if self._per_tensor or len(steps) != 1:   # parameters with different step counts (some had no gradient earlier): per tensor
+        if len(steps) != 1:   # parameters with different step counts (some had no gradient earlier): per tensor
             for p in live:
                 st = self.state[p]
                 st["step"] += 1

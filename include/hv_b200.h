@@ -374,18 +374,13 @@ int hv_resample_curve(const double* vol, int d0, int d1, int d2, const double* k
 
 /* ======================================================================================
  * Debug / measurement hooks.  NOT part of the drop-in surface: no reference interface stands behind them; they only
- * make the library's own kernels observable (tools/trace_conv.py, tools/timeline_forward.py, tools/trace_trunk.py).
+ * make the library's own kernels observable (tools/trace_conv.py, tools/timeline_forward.py).
  * dev_buf = NULL switches a hook off.
  * ==================================================================================== */
 /* CTA 0 of every subsequent conv_tc launch appends (tag, clock64) stamps per role: dev_buf = 12000 + 4 * 400 int64 */
 int hv_debug_conv_trace(void* dev_buf);
 /* conv_tc launch i (host launch order) records {first CTA entry, last CTA exit} globaltimer ns at dev_buf[4 i], [4 i + 1] */
 int hv_debug_conv_timeline(void* dev_buf);
-/* CTA `cta` of every subsequent trunk_tc launch appends (tag, item, clock64) stamps per role: dev_buf = 12000 int64 */
-int hv_debug_trunk_trace(void* dev_buf, int cta);
-/* A/B switch of the bf16 conv backward: bit 0 = data gradient through the GEMM + col2im path for every layer, bit 1 = weight
- * gradient through the explicit im2col operand for every layer (0: the shifted-operand paths where they apply)            */
-int hv_debug_backward_paths(int bits);
 
 #ifdef __cplusplus
 }

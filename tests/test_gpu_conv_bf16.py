@@ -226,28 +226,3 @@ def test_every_plan_instance_against_bf16_rounded_torch(gen_bf16, synthetic_sd, 
             _close(got, want, full, rounded=not head)
         prev = full
 
-
-def test_dataflow_trunk_kernel_passes_the_plan_instance_check():
-    """The dataflow trunk kernel (csrc/trunk_tc.cu: chains of 64 -> 64 layers as ONE launch) is opt-in (HV_TRUNK=1, read once per
-    process): the per-instance check above must hold with it, and the forward must be bit-identical to the per-layer launches."""
-    import os
-    import subprocess
-    import sys
-    if os.environ.get("HV_TRUNK") == "1":
-        pytest.skip("already inside the HV_TRUNK=1 run")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, HV_TRUNK="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_conv_bf16.py"), "-q", "-m", "gpu", "-k",
-                        "every_plan_instance", "-p", "no:cacheprovider"], env=env, cwd=root, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    code = ("import torch, sys; sys.path.insert(0, %r); import healthivert_gan_b200 as hv; from oracle import synth;"
-            "g = hv.Generator({'input_dim': 1, 'ngf': 16}, True); g.load_state_dict(synth.synthetic_generator_state_dict());"
-            "g = g.cuda().eval(); g.precision = 'bf16';"
-            "o = g(*[t.cuda() for t in synth.synthetic_slices(16, seed=8)]); torch.cuda.synchronize();"
-            "print('SUM', float(o[3].double().sum()), float(o[1].double().sum()))" % root)
-    sums = []
-    for trunk in ("0", "1"):
-        r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, HV_TRUNK=trunk), cwd=root, capture_output=True, text=True, timeout=600)
-        assert r.returncode == 0, r.stderr[-2000:]
-        sums.append([l for l in r.stdout.splitlines() if l.startswith("SUM")][-1])
-    assert sums[0] == sums[1], sums

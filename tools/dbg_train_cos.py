@@ -8,15 +8,13 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 
-from healthivert_gan_b200 import _lib
 from healthivert_gan_b200.pix2pix_model import Pix2PixModel
 from oracle import synth
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 2
 
 
-def grads(precision, g_forward, paths):
-    _lib.lib().hv_debug_backward_paths(paths)
+def grads(precision, g_forward):
     opt = synth.train_options(gpu_ids=[0], precision=precision, g_forward_precision=g_forward)
     m = Pix2PixModel(opt)
     m.setup(opt)
@@ -30,9 +28,8 @@ def grads(precision, g_forward, paths):
     return {k: p.grad.double().flatten().clone() for k, p in m.netG.named_parameters()}
 
 
-ref = grads("fp32", "fp32", 0)
-for label, args in (("bf16 backward, GEMM dgrad + im2col wgrad", ("bf16", "fp32", 3)), ("bf16 backward, conv dgrad + im2col wgrad", ("bf16", "fp32", 2)),
-                    ("bf16 backward, conv dgrad + shifted wgrad", ("bf16", "fp32", 0)), ("bf16 forward + backward (new paths)", ("bf16", "bf16", 0))):
+ref = grads("fp32", "fp32")
+for label, args in (("bf16 backward (fp32 forward)", ("bf16", "fp32")), ("bf16 forward + backward", ("bf16", "bf16"))):
     g = grads(*args)
     rows = []
     for k in ref:

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """One golden training step (n = 2) in the tensor-core mode: gradient-norm deviations and gradient direction against the golden
-vectors of the unmodified reference.  Environment switches (HV_DGRAD_GEMM, HV_WGRAD_IM2COL) and --g-forward select the kernels."""
+vectors of the unmodified reference.  --g-forward selects the precision of the generator's forward."""
 import argparse
 import os
 import sys

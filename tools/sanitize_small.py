@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Smallest run that touches every new round-2 kernel family once (for `compute-sanitizer --tool memcheck`): bf16 forward (sub-pixel
-upsample instances, split input packing), the uint8 pipeline with its CUDA graph, the dataflow trunk kernel (HV_TRUNK=1 run separately),
-the fused post-forward kernel and one training step in the tensor-core mode (dconv / gconv GEMM paths, multi-tensor Adam)."""
+upsample instances, split input packing), the uint8 pipeline with its CUDA graph, the fused post-forward kernel and one training
+step in the tensor-core mode (dconv / gconv GEMM paths, multi-tensor Adam)."""
 import os
 import sys
 
