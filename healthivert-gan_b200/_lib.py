@@ -72,6 +72,9 @@ SIGNATURES = {
                                 c_void_p]),
     "hv_bn_lrelu_fwd": (c_int, [c_void_p] * 8 + [c_int, c_int, c_int, c_float, c_float, c_float, c_void_p]),
     "hv_bn_lrelu_bwd": (c_int, [c_void_p] * 9 + [c_int, c_int, c_int, c_float, c_void_p]),
+    "hv_in_lrelu_fwd": (c_int, [c_void_p] * 5 + [c_int, c_int, c_int, c_float, c_float, c_void_p]),
+    "hv_in_lrelu_bwd": (c_int, [c_void_p] * 7 + [c_int, c_int, c_int, c_float, c_void_p]),
+    "hv_act_fwd": (c_int, [c_void_p, c_void_p, c_int, c_size_t, c_void_p]),
     "hv_reduce_scalar": (c_int, [c_void_p, c_void_p, c_float, c_int, c_size_t, c_float, c_void_p, c_void_p, c_void_p]),
     "hv_loss_grad": (c_int, [c_void_p, c_void_p, c_float, c_int, c_float, c_void_p, c_int, c_void_p, c_int, c_size_t,
                              c_void_p]),

@@ -1,9 +1,12 @@
 """Drop-in mirror of the hot-path parts of the reference's ``models/networks.py`` on hand-written kernels:
 ``NLayerDiscriminator`` (:555-602), ``GANLoss`` (:212-278, vanilla / BCE-with-logits), ``define_D`` (:163-206),
-``init_weights`` / ``init_net`` (:68-117), ``get_scheduler`` ('linear', :52-56).
+``get_norm_layer`` (:30-47: 'batch', 'instance', 'none'), ``Identity`` (:25-27), ``init_weights`` / ``init_net`` (:68-117),
+``get_scheduler`` ('linear', :52-56).
 
-The torch ``nn.Conv2d`` / ``nn.BatchNorm2d`` objects are parameter CONTAINERS only (identical ``state_dict`` keys
-``model.{0,2,3,5,6,8,9,11}.*`` and identical initialisation streams); all arithmetic runs in libhv_b200.so.
+The torch ``nn.Conv2d`` / ``nn.BatchNorm2d`` objects are parameter CONTAINERS only (identical ``state_dict`` keys and identical
+initialisation streams); all arithmetic runs in libhv_b200.so.  Discriminator layouts by norm:
+'batch' ``model.{0,2,3,5,6,8,9,11}.*``; 'instance' ``model.{0,2,5,8,11}.{weight,bias}`` (InstanceNorm2d(affine=False) has no
+state, the convs before it have a bias); 'none' ``model.{0,11}.{weight,bias}`` + ``model.{2,5,8}.weight``.
 """
 import functools
 
@@ -15,15 +18,27 @@ from . import _lib, train_ops as T
 from ._lib import HV_SRC_DIRECT
 
 
+class Identity(nn.Module):
+    def forward(self, x):
+        return x
+
+
 def get_norm_layer(norm_type="batch"):
     if norm_type == "batch":
         return functools.partial(nn.BatchNorm2d, affine=True, track_running_stats=True)
-    raise NotImplementedError("normalization layer [%s] is not built (the path uses 'batch')" % norm_type)
+    if norm_type == "instance":
+        return functools.partial(nn.InstanceNorm2d, affine=False, track_running_stats=False)
+    if norm_type == "none":
+        def norm_layer(x):
+            return Identity()
+        return norm_layer
+    raise NotImplementedError("normalization layer [%s] is not found" % norm_type)
 
 
 class NLayerDiscriminator(nn.Module):
-    """PatchGAN discriminator (reference models/networks.py:555-602): conv4x4 s2 + LReLU, (conv4x4 s2 + BN + LReLU) x2,
-    conv4x4 s1 + BN + LReLU, conv4x4 s1 -> 1-channel logits."""
+    """PatchGAN discriminator (reference models/networks.py:555-602): conv4x4 s2 + LReLU, (conv4x4 s2 + norm + LReLU) x2,
+    conv4x4 s1 + norm + LReLU, conv4x4 s1 -> 1-channel logits.  norm: BatchNorm2d (train mode only), InstanceNorm2d(affine=False)
+    (fused with the LeakyReLU, train and eval) or Identity (the LeakyReLU is fused into the conv)."""
 
     def __init__(self, input_nc, ndf=64, n_layers=3, norm_layer=nn.BatchNorm2d):
         super().__init__()
@@ -43,8 +58,9 @@ class NLayerDiscriminator(nn.Module):
                      norm_layer(ndf * nf_mult), nn.LeakyReLU(0.2, True)]
         sequence += [nn.Conv2d(ndf * nf_mult, 1, kernel_size=kw, stride=1, padding=padw)]
         self.model = nn.Sequential(*sequence)
-        # 'fp32': SIMT parity kernels everywhere; 'bf16': the BatchNorm-followed 4x4 convs (64->128, 128->256, 256->512: 97 % of the
-        # discriminator's FLOPs) run on the tensor cores with bf16 operands and fp32 accumulation (train_ops.conv2d_tc)
+        # 'fp32': SIMT parity kernels everywhere; 'bf16': the three 4x4 convs between the first and the last (64->128, 128->256,
+        # 256->512: 97 % of the discriminator's FLOPs) run on the tensor cores with bf16 operands and fp32 accumulation
+        # (train_ops.conv2d_tc)
         self.precision = "fp32"
 
     def run(self, x, tape=None, param_grads=True):
@@ -59,8 +75,15 @@ class NLayerDiscriminator(nn.Module):
             m = mods[i]
             if not isinstance(m, nn.Conv2d):
                 raise NotImplementedError("unexpected module in the PatchGAN sequence: %r" % (m,))
-            nxt = mods[i + 1] if i + 1 < len(mods) else None
-            fused_lrelu = isinstance(nxt, nn.LeakyReLU)
+            # the reference's blocks: conv [-> BatchNorm2d | InstanceNorm2d | Identity] [-> LeakyReLU(0.2)]
+            j = i + 1
+            norm = mods[j] if j < len(mods) and isinstance(mods[j], (nn.BatchNorm2d, nn.InstanceNorm2d, Identity)) else None
+            j += norm is not None
+            lrelu = j < len(mods) and isinstance(mods[j], nn.LeakyReLU)
+            if isinstance(norm, nn.InstanceNorm2d) and (norm.affine or norm.track_running_stats or not lrelu):
+                raise NotImplementedError("hv_b200 NLayerDiscriminator: InstanceNorm2d is built as get_norm_layer('instance') makes it")
+            inorm = isinstance(norm, nn.InstanceNorm2d)
+            bare_lrelu = lrelu and not isinstance(norm, (nn.BatchNorm2d, nn.InstanceNorm2d))   # conv [-> Identity] -> LeakyReLU
             w = m.weight.detach()
             b = m.bias.detach() if m.bias is not None else None
 
@@ -70,19 +93,25 @@ class NLayerDiscriminator(nn.Module):
                     T.accumulate_param(m.bias, db)
 
             h, wd = x.data.shape[2], x.data.shape[3]
-            tc = (self.precision == "bf16" and b is None and not fused_lrelu and m.kernel_size == (4, 4) and m.padding == (1, 1)
-                  and m.dilation == (1, 1) and m.stride[0] in (1, 2) and m.in_channels % 8 == 0 and m.out_channels % 128 == 0)
+            # the tensor cores take the normalised or norm-free 4x4 convs (64->128, 128->256, 256->512: 97 % of the FLOPs); a bias
+            # before InstanceNorm goes into the norm kernel
+            tc = (self.precision == "bf16" and norm is not None and (b is None or inorm) and m.kernel_size == (4, 4)
+                  and m.padding == (1, 1) and m.dilation == (1, 1) and m.stride[0] in (1, 2) and m.in_channels % 8 == 0
+                  and m.out_channels % 128 == 0)
             if tc:
                 x = T.conv2d_tc(tape, x, w.contiguous(), m.stride[0], on_grad, param_grads)
+                if bare_lrelu:
+                    x = T.lrelu(tape, x)
             else:
                 x = T.conv2d(tape, [(x, HV_SRC_DIRECT)], w, b, m.kernel_size[0], m.stride[0], m.padding[0], m.dilation[0],
-                             "lrelu" if fused_lrelu else "none", (h, wd), on_grad, param_grads)
-            i += 2 if fused_lrelu else 1
-            if i < len(mods) and isinstance(mods[i], nn.BatchNorm2d):
+                             "lrelu" if bare_lrelu else "none", (h, wd), on_grad, param_grads)
+            if isinstance(norm, nn.BatchNorm2d):
                 if not self.training:
                     raise NotImplementedError("hv_b200 NLayerDiscriminator: eval-mode BatchNorm is not on the training path")
-                x = T.bn_lrelu(tape, x, mods[i], 0.2, param_grads)
-                i += 2  # BatchNorm2d + LeakyReLU
+                x = T.bn_lrelu(tape, x, norm, 0.2, param_grads)
+            elif inorm:
+                x = T.in_lrelu(tape, x, m.bias if tc else None, 0.2, norm.eps, param_grads)
+            i = j + 1 if lrelu else j
         return x
 
     def forward(self, input):

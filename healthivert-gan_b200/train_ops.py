@@ -327,6 +327,56 @@ def bn_lrelu(tape, x, bn, slope=0.2, param_grads=True):
     return out
 
 
+def in_lrelu(tape, x, bias=None, slope=0.2, eps=1e-5, param_grads=True):
+    """InstanceNorm2d(affine=False) + LeakyReLU(slope) (reference networks.py:583-597 with norm='instance'), instance statistics in
+    train and eval.  bias: the preceding convolution's bias parameter, added on load (the tensor-core conv has no bias epilogue); its
+    gradient, zero up to rounding, is accumulated into bias.grad when param_grads."""
+    n, c, h, w = x.data.shape
+    dev = x.data.device
+    y = torch.empty_like(x.data)
+    mean = torch.empty(n * c, device=dev, dtype=torch.float32)
+    invstd = torch.empty(n * c, device=dev, dtype=torch.float32)
+    b = bias.detach() if bias is not None else None
+    check(_L().hv_in_lrelu_fwd(ptr(x.data), ptr(b), ptr(y), ptr(mean), ptr(invstd), n, c, h * w, float(eps), float(slope),
+                               _lib.stream()))
+    out = Var(y)
+    if tape is None:
+        return out
+
+    def bwd():
+        if out.grad is None:
+            return
+        dx = torch.empty_like(x.data)
+        db = torch.empty(c, device=dev, dtype=torch.float32) if (b is not None and param_grads) else None
+        check(_L().hv_in_lrelu_bwd(ptr(x.data), ptr(b), ptr(out.grad.contiguous()), ptr(mean), ptr(invstd), ptr(dx), ptr(db), n, c,
+                                   h * w, float(slope), _lib.stream()))
+        if db is not None:
+            accumulate_param(bias, db)
+        accumulate(x, dx)
+
+    tape.record(bwd)
+    return out
+
+
+def lrelu(tape, x):
+    """LeakyReLU(0.2) as its own pass (after a tensor-core convolution, which has no activation epilogue)."""
+    y = torch.empty_like(x.data)
+    check(_L().hv_act_fwd(ptr(x.data), ptr(y), HV_ACT["lrelu"], y.numel(), _lib.stream()))
+    out = Var(y)
+    if tape is None:
+        return out
+
+    def bwd():
+        if out.grad is None:
+            return
+        dx = torch.empty_like(y)
+        check(_L().hv_act_bwd(ptr(y), ptr(out.grad.contiguous()), ptr(dx), HV_ACT["lrelu"], y.numel(), _lib.stream()))
+        accumulate(x, dx)
+
+    tape.record(bwd)
+    return out
+
+
 # ------------------------------------------------------------------------------------------- scalar losses
 class Scratch:
     """Per-device reduction scratch (1024 floats) and 0-dim outputs."""

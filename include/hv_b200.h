@@ -277,6 +277,19 @@ int hv_bn_lrelu_fwd(const float* x, const float* gamma, const float* beta, float
 int hv_bn_lrelu_bwd(const float* x, const float* y, const float* dy, const float* gamma, const float* save_mean,
                     const float* save_invstd, float* dx, float* dgamma, float* dbeta, int n, int c, int hw,
                     float slope, hv_stream_t stream);
+/* ---- A7 with norm='instance': InstanceNorm2d(affine=False) + LeakyReLU(slope) per (sample, channel) plane of x [n,c,hw]
+ * (models/networks.py:555-602 with get_norm_layer('instance')): y = lrelu((x + bias[c] - mean) / sqrt(var + eps)), biased variance
+ * over hw, instance statistics in train and eval alike.  bias [c] (the preceding convolution's, added on load) may be NULL.
+ * save_mean / save_invstd [n*c] feed the backward.  8 bytes per element when hw <= 4096 (the plane stays on chip).
+ * bwd: dx from x, dy and the saved statistics (12 bytes per element when hw <= 4096); dbias [c] = sum over (n, hw) of dx (the
+ * gradient of the bias added on load; may be NULL; zero up to rounding).  Larger planes stream x (and dy) twice.                  */
+int hv_in_lrelu_fwd(const float* x, const float* bias, float* y, float* save_mean, float* save_invstd, int n, int c, int hw,
+                    float eps, float slope, hv_stream_t stream);
+int hv_in_lrelu_bwd(const float* x, const float* bias, const float* dy, const float* save_mean, const float* save_invstd,
+                    float* dx, float* dbias, int n, int c, int hw, float slope, hv_stream_t stream);
+/* y = act(x) elementwise (act: HV_ACT_NONE .. HV_ACT_CLAMP1; y may equal x): the LeakyReLU after a tensor-core convolution of the
+ * norm-free PatchGAN (norm='none'); its backward is hv_act_bwd.                                                                   */
+int hv_act_fwd(const float* x, float* y, int act, size_t count, hv_stream_t stream);
 
 /* ---- A6: scalar losses.  out[0] = scale * reduce; kind 0: sum|a-b| (nn.L1Loss), 1: BCE-with-logits
  * against the constant target t (GANLoss vanilla, models/networks.py:237,:270-272), 2: count_nonzero(a)
