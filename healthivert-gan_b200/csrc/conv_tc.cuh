@@ -206,6 +206,32 @@ void tc_tail_set_outputs(TcTail& t, float* head0, float* head1);
 // also write head 1 as tc_pack_kx(k = 5, dil = 1) would into chunk `chunk` of dst (null: off)
 int tc_tail_set_kxpack(TcTail& t, const TcBuf* dst, int chunk);
 int tc_tail_launch(const TcTail& t, cudaStream_t st);
+// fused input stem of a generator stage (stem_tc.cu): the kx-packed 5x5 input conv and the stride-2 conv(s) that read its output in one
+// persistent launch; the 256 x 256 intermediate stays in shared memory
+struct TcStemParams {
+  CUtensorMap map_in;    // input rows of the 5x5 conv: {half-row position, half, plane row, chunk, image}
+  const void* w1;        // packed weights / padded bias of the per-layer instances (TcConv::w_packed, bias_pad): 5x5 conv,
+  const void* w2;        // stride-2 conv on intermediate chunks 0-1, and (fine stage) the one on chunks 2-3
+  const void* w3;
+  const float* bias1;
+  const float* bias2;
+  const float* bias3;
+  __nv_bfloat16* out2;   // outputs of the stride-2 convs (plain chunked 128 x 128 buffers of one geometry)
+  __nv_bfloat16* out3;
+  int out2_chunks, out3_chunks, out_pitch, out_border, out_plane;
+  int n, rows_per_unit, strips, units;   // work unit = (image, strip of rows_per_unit stride-2 output rows)
+  long long* timeline;
+};
+struct TcStem {
+  TcStemParams p;
+  int grid = 0;
+  bool fine = false;
+};
+// conv1: the kx-packed 5x5 conv (space-to-depth output); down: the stride-2 conv on its chunks 0-1; down2 (fine stage): the stride-2
+// conv on chunks 2-3, or null.  The weights are read from the instances' packed buffers at launch time.
+int tc_stem_setup(TcStem& s, const TcConv& conv1, const TcConv& down, const TcConv* down2, int n_images);
+void tc_stem_set_batch(TcStem& s, int n_images);
+int tc_stem_launch(const TcStem& s, cudaStream_t st);
 // next slot of the timeline hook (or null), shared with conv_tc.cu
 long long* tc_timeline_next();
 

@@ -284,11 +284,21 @@ struct TcPlan {
   // the 16 -> 8 conv + dual heads of each stage as ONE launch (tail_tc.cu): conv16 -> conv17 | conv18, allconv16 -> allconv17 | allconv18
   TcTail tail[2];
   bool tail_fused_last = false;        // the last forward ran the fused tails: B_C16 / chunk 0 of B_A16CAT were not written
+  // the 5x5 input conv + the stride-2 conv(s) after it as ONE launch per stage (stem_tc.cu): conv1 -> conv2_downsample,
+  // conv1 | pmconv1 -> conv2_downsample, pmconv2_downsample
+  TcStem stem[2];
+  bool stem_fused_last = false;        // the last forward ran the fused stems: B_C1 / B_F1 (and its view B_P1) were not written
 };
 
 // HV_NO_TAIL_FUSE=1: the per-layer launches for the thin tails (A/B runs, parity tests); read once per process.
 static bool tail_fuse_enabled() {
   static const bool on = !(getenv("HV_NO_TAIL_FUSE") && atoi(getenv("HV_NO_TAIL_FUSE")) != 0);
+  return on;
+}
+
+// HV_NO_STEM_FUSE=1: the per-layer launches for the input stems (reference of the parity test); read once per process.
+static bool stem_fuse_enabled() {
+  static const bool on = !(getenv("HV_NO_STEM_FUSE") && atoi(getenv("HV_NO_STEM_FUSE")) != 0);
   return on;
 }
 
@@ -367,6 +377,11 @@ static int tc_plan_create(hv_generator* g) {
     if (!rc) rc = tc_tail_set_kxpack(t->tail[0], &t->buf[B_IN_F], 2);
     if (rc) return rc;
   }
+  if (stem_fuse_enabled()) {
+    int rc = tc_stem_setup(t->stem[0], t->conv[C1], t->conv[C2], nullptr, n);
+    if (!rc) rc = tc_stem_setup(t->stem[1], t->conv[F1], t->conv[F2], &t->conv[PM2], n);
+    if (rc) return rc;
+  }
   return HV_OK;
 }
 
@@ -426,8 +441,16 @@ static int forward_bf16(hv_generator* g, const float* x, const float* mask, cons
     RC(tc_pack_kx(in_f0, 3, 5, 1, view(B_IN_F).chunk_view(0, 2), ax));
     if (use_aux) HV_CUDA(cudaEventRecord(g->ev_aux[1], ax));
   }
+  const bool fuse_stem = stem_fuse_enabled();
+  // the 5x5 input conv of a stage and the stride-2 conv(s) after it: one fused launch (stem_tc.cu), or the per-layer launches
+  auto stem = [&](int which) -> int {
+    tc_stem_set_batch(t->stem[which], n);
+    return tc_stem_launch(t->stem[which], st);
+  };
   // ---- coarse network
-  for (int l : {C1, C2, C3, C4, C5, C6, C7, C8, C9, C10, C11, C12}) RC(run(l, st));
+  if (fuse_stem) RC(stem(0));
+  else for (int l : {C1, C2}) RC(run(l, st));
+  for (int l : {C3, C4, C5, C6, C7, C8, C9, C10, C11, C12}) RC(run(l, st));
   RC(fork_aux(2));   // the height head reads conv10_atrous (:90-93); nothing of the trunk overwrites it
   RC(tc_gap_fc_sigmoid(view(B_C10), g->fc_w[0], g->fc_b[0], pred1_h, t->gap_partial, t->gap_ticket, ax));
   if (use_aux) HV_CUDA(cudaStreamWaitEvent(st, g->ev_aux[1], 0));
@@ -451,16 +474,20 @@ static int forward_bf16(hv_generator* g, const float* x, const float* mask, cons
     const TcPlaneSrc in_f1[1] = {{coarse_seg, HV_SRC_DIRECT}};   // chunks 2-3: the only part packed on the critical path
     RC(tc_pack_kx(in_f1, 1, 5, 1, view(B_IN_F).chunk_view(2, 2), st));
   }
-  RC(run(F1, st));
+  // the fused fine stem also runs pmconv2: the attention branch then starts at pmconv3
+  if (fuse_stem) RC(stem(1));
+  else RC(run(F1, st));
   HV_CUDA(cudaEventRecord(g->ev_fork, st));
   HV_CUDA(cudaStreamWaitEvent(g->side, g->ev_fork, 0));
   cudaStream_t sa = g->side;
-  for (int l : {PM2, PM3, PM4, PM5, PM6}) RC(run(l, sa));
+  if (!fuse_stem) RC(run(PM2, sa));
+  for (int l : {PM3, PM4, PM5, PM6}) RC(run(l, sa));
   RC(ctx_attn_fwd_tc(view(B_P6), mask, view(B_CA), offsets, flow, 10.f, 1, per_sample_mask, t->ca_ws, sa, use_aux ? ax : nullptr,
                      use_aux ? &g->ev_aux[6] : nullptr));
   for (int l : {PM9, PM10}) RC(run(l, sa));
   HV_CUDA(cudaEventRecord(g->ev_join, sa));
-  for (int l : {F2, F3, F4, F5, F6, F7, F8, F9, F10}) RC(run(l, st));
+  if (!fuse_stem) RC(run(F2, st));
+  for (int l : {F3, F4, F5, F6, F7, F8, F9, F10}) RC(run(l, st));
   HV_CUDA(cudaStreamWaitEvent(st, g->ev_join, 0));
   RC(run(A11, st));
   RC(fork_aux(4));
@@ -468,6 +495,7 @@ static int forward_bf16(hv_generator* g, const float* x, const float* mask, cons
   for (int l : {A12, A19, A13, A14, A15}) RC(run(l, st));
   RC(tail(1, A16, A17, x_stage2, fine_seg));
   t->tail_fused_last = fuse_tail;
+  t->stem_fused_last = fuse_stem;
   RC(join_aux(5));
   g->last_heads[0] = x_stage1; g->last_heads[1] = coarse_seg; g->last_heads[2] = x_stage2; g->last_heads[3] = fine_seg;
   g->last_n = n;
@@ -659,6 +687,14 @@ long long hv_generator_read_tap(hv_generator* g, int idx, float* out, hv_stream_
         // (B_C15 / B_A15), which the forward leaves intact
         tc_set_batch(g->tc->conv[idx], g->last_n);
         int rc = tc_conv_launch(g->tc->conv[idx], as_stream(stream));
+        if (rc) return rc;
+      }
+      if (g->tc->stem_fused_last && (idx == C1 || idx == F1 || idx == PM1)) {
+        // the fused stem kept this layer's output in shared memory: recompute it with the per-layer instance (the merged conv1 | pmconv1
+        // for F1 and PM1) from its input (B_IN_C / B_IN_F), which the forward leaves intact
+        TcConv& c = g->tc->conv[idx == C1 ? C1 : F1];
+        tc_set_batch(c, g->last_n);
+        int rc = tc_conv_launch(c, as_stream(stream));
         if (rc) return rc;
       }
       const int ch = idx == A16 ? 8 : kLayers[idx].cout;
