@@ -696,7 +696,7 @@ int bn_lrelu_bwd(const float* x, const float* y, const float* dy, const float* g
 
 // ------------------------------------------------------------------ scalar losses (two-stage deterministic reductions)
 // kind: 0 sum|a-b|  1 BCE-with-logits vs constant target t (a = logits, b unused)  2 count_nonzero(a)
-//       3 sum a  4 sum a*b
+//       3 sum a  4 sum a*b  5 sum (a-t)^2 (b unused)
 __global__ void __launch_bounds__(256) reduce_partial_kernel(const float* __restrict__ a, const float* __restrict__ b, float t, int kind,
                                                              size_t count, float* __restrict__ partial) {
   __shared__ float red[32];
@@ -708,7 +708,8 @@ __global__ void __launch_bounds__(256) reduce_partial_kernel(const float* __rest
       case 1: s += fmaxf(x, 0.f) - x * t + log1pf(expf(-fabsf(x))); break;
       case 2: s += x != 0.f ? 1.f : 0.f; break;
       case 3: s += x; break;
-      default: s += x * b[i];
+      case 4: s += x * b[i]; break;
+      case 5: { const float d = x - t; s += d * d; } break;
     }
   }
   s = block_sum(s, red);
@@ -725,7 +726,8 @@ __global__ void __launch_bounds__(256) reduce_final_kernel(const float* __restri
 
 // out[0] = scale * reduce(kind);  scratch: 1024 floats
 int reduce_scalar(const float* a, const float* b, float t, int kind, size_t count, float scale, float* out, float* scratch, cudaStream_t st) {
-  HV_CHECK_ARG(a && out && scratch && (kind == 1 || kind == 2 || kind == 3 || b), "reduce_scalar: null argument");
+  HV_CHECK_ARG(kind >= 0 && kind <= 5, "reduce_scalar: kind %d is not one of 0..5", kind);
+  HV_CHECK_ARG(a && out && scratch && ((kind != 0 && kind != 4) || b), "reduce_scalar: null argument");
   int blocks = (int)((count + 255) / 256);
   if (blocks > 1024) blocks = 1024;
   if (blocks < 1) blocks = 1;
@@ -736,8 +738,9 @@ int reduce_scalar(const float* a, const float* b, float t, int kind, size_t coun
   return HV_OK;
 }
 
-// gradients of the elementwise losses.  kind 0: da = scale[0] * g * sign(a - b);  kind 1: da = g * (sigmoid(a) - t)
-// (`scale` is an optional DEVICE scalar multiplier, e.g. 256*256 / count_nonzero(mask); accumulate adds into da)
+// gradients of the elementwise losses, gg = g * S:  kind 0: da = gg * sign(a - b);  1: da = gg * (sigmoid(a) - t);
+// 2: da = gg * 2 (a - t);  3: da = gg (a is not read).  S = 1, scale[0] or 1 / scale[0]: `scale` is an
+// optional DEVICE scalar multiplier, e.g. 256*256 / count_nonzero(mask); accumulate adds into da
 __global__ void loss_grad_kernel(const float* __restrict__ a, const float* __restrict__ b, float t, int kind, float g, const float* __restrict__ scale,
                                  int scale_is_reciprocal, float* __restrict__ da, int accumulate, size_t count) {
   float gg = g;
@@ -746,15 +749,20 @@ __global__ void loss_grad_kernel(const float* __restrict__ a, const float* __res
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   for (; i < count; i += stride) {
     float d;
-    if (kind == 0) { const float df = a[i] - b[i]; d = df > 0.f ? gg : (df < 0.f ? -gg : 0.f); }
-    else d = gg * (1.f / (1.f + expf(-a[i])) - t);
+    switch (kind) {
+      case 0: { const float df = a[i] - b[i]; d = df > 0.f ? gg : (df < 0.f ? -gg : 0.f); } break;
+      case 1: d = gg * (1.f / (1.f + expf(-a[i])) - t); break;
+      case 2: d = gg * (2.f * (a[i] - t)); break;
+      default: d = gg; break;   // 3 (loss_grad checks the range)
+    }
     da[i] = accumulate ? da[i] + d : d;
   }
 }
 
 int loss_grad(const float* a, const float* b, float t, int kind, float g, const float* scale, int scale_is_reciprocal, float* da,
               int accumulate, size_t count, cudaStream_t st) {
-  HV_CHECK_ARG(a && da && (kind == 1 || b), "loss_grad: null argument");
+  HV_CHECK_ARG(kind >= 0 && kind <= 3, "loss_grad: kind %d is not one of 0..3", kind);
+  HV_CHECK_ARG(a && da && (kind != 0 || b), "loss_grad: null argument");
   loss_grad_kernel<<<ew_blocks(count), 256, 0, st>>>(a, b, t, kind, g, scale, scale_is_reciprocal, da, accumulate, count);
   HV_LAUNCH_CHECK();
   return HV_OK;

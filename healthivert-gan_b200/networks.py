@@ -1,7 +1,8 @@
 """Drop-in mirror of the hot-path parts of the reference's ``models/networks.py`` on hand-written kernels:
-``NLayerDiscriminator`` (:555-602), ``GANLoss`` (:212-278, vanilla / BCE-with-logits), ``define_D`` (:163-206),
-``get_norm_layer`` (:30-47: 'batch', 'instance', 'none'), ``Identity`` (:25-27), ``init_weights`` / ``init_net`` (:68-117),
-``get_scheduler`` ('linear', :52-56).
+``NLayerDiscriminator`` (:555-602), ``GANLoss`` (:212-278: 'vanilla', 'lsgan', 'wgangp' without a gradient penalty),
+``define_D`` (:163-206), ``get_norm_layer`` (:30-47: 'batch', 'instance', 'none'), ``Identity`` (:25-27),
+``init_weights`` / ``init_net`` (:68-117), ``get_scheduler`` (:39-65: 'linear', 'step', 'plateau', 'cosine', torch's own
+schedulers on ``train_ops.FusedAdam``).
 
 The torch ``nn.Conv2d`` / ``nn.BatchNorm2d`` objects are parameter CONTAINERS only (identical ``state_dict`` keys and identical
 initialisation streams); all arithmetic runs in libhv_b200.so.  Discriminator layouts by norm:
@@ -13,6 +14,7 @@ import functools
 import torch
 import torch.nn as nn
 from torch.nn import init
+from torch.optim import lr_scheduler
 
 from . import _lib, train_ops as T
 from ._lib import HV_SRC_DIRECT
@@ -119,21 +121,35 @@ class NLayerDiscriminator(nn.Module):
 
 
 class GANLoss(nn.Module):
-    """reference models/networks.py:212-278; only the 'vanilla' objective (BCEWithLogitsLoss) is on the path."""
+    """reference models/networks.py:212-278.  'vanilla': BCEWithLogitsLoss and 'lsgan': MSELoss against the constant real / fake
+    label; 'wgangp': -mean(prediction) against real, mean(prediction) against fake.  The reference's pix2pix model never calls
+    cal_gradient_penalty, so 'wgangp' has no gradient penalty (and no weight clipping) here either.
+
+    ``__call__`` returns the loss as a 0-dim device tensor; ``grad(prediction, target_is_real, g)`` returns d(g * loss)/d prediction."""
 
     def __init__(self, gan_mode, target_real_label=1.0, target_fake_label=0.0):
         super().__init__()
         self.register_buffer("real_label", torch.tensor(target_real_label))
         self.register_buffer("fake_label", torch.tensor(target_fake_label))
         self.gan_mode = gan_mode
-        if gan_mode != "vanilla":
+        if gan_mode not in T.GAN_KINDS:
             raise NotImplementedError("gan mode %s not implemented" % gan_mode)
+        # the kernels take the target by value: kept as Python floats, so no call reads the buffers back from the device
+        self._labels = (float(target_fake_label), float(target_real_label))
+
+    def _target(self, target_is_real):
+        """(t, sign) of train_ops.gan_loss"""
+        if self.gan_mode == "wgangp":
+            return 0.0, (-1.0 if target_is_real else 1.0)
+        return self._labels[bool(target_is_real)], 1.0
 
     def __call__(self, prediction, target_is_real):
-        return T.bce_logits_const(prediction, target_is_real)[0]
+        t, sign = self._target(target_is_real)
+        return T.gan_loss(prediction, self.gan_mode, t, sign)[0]
 
     def grad(self, prediction, target_is_real, g=1.0):
-        return T.bce_logits_const_grad(prediction.contiguous(), target_is_real, g)
+        t, sign = self._target(target_is_real)
+        return T.gan_loss_grad(prediction.contiguous(), self.gan_mode, t, g, sign)
 
 
 def init_weights(net, init_type="normal", init_gain=0.02):
@@ -180,21 +196,17 @@ def define_D(input_nc, ndf, netD, n_layers_D=3, norm="batch", init_type="normal"
     return init_net(net, init_type, init_gain, gpu_ids)
 
 
-class LinearLR:
-    """'linear' policy of get_scheduler (reference :52-56) for FusedAdam."""
-
-    def __init__(self, optimizer, opt):
-        self.optimizer, self.opt, self.epoch = optimizer, opt, 0
-
-    def step(self):
-        self.epoch += 1
-        o = self.opt
-        f = 1.0 - max(0, self.epoch + o.epoch_count - o.n_epochs) / float(o.n_epochs_decay + 1)
-        for g in self.optimizer.param_groups:
-            g["lr"] = g["initial_lr"] * f
-
-
 def get_scheduler(optimizer, opt):
+    """reference models/networks.py:39-65: torch's own schedulers (train_ops.FusedAdam is a torch.optim.Optimizer).  'plateau' is
+    stepped with the model's metric (BaseModel.update_learning_rate); opt.lr_decay_iters is read by 'step' alone."""
     if opt.lr_policy == "linear":
-        return LinearLR(optimizer, opt)
+        def lambda_rule(epoch):
+            return 1.0 - max(0, epoch + opt.epoch_count - opt.n_epochs) / float(opt.n_epochs_decay + 1)
+        return lr_scheduler.LambdaLR(optimizer, lr_lambda=lambda_rule)
+    if opt.lr_policy == "step":
+        return lr_scheduler.StepLR(optimizer, step_size=opt.lr_decay_iters, gamma=0.1)
+    if opt.lr_policy == "plateau":
+        return lr_scheduler.ReduceLROnPlateau(optimizer, mode="min", factor=0.2, threshold=0.01, patience=5)
+    if opt.lr_policy == "cosine":
+        return lr_scheduler.CosineAnnealingLR(optimizer, T_max=opt.n_epochs, eta_min=0)
     raise NotImplementedError("learning rate policy [%s] is not implemented" % opt.lr_policy)

@@ -57,7 +57,10 @@ class BaseModel:
     def update_learning_rate(self):
         old_lr = self.optimizers[0].param_groups[0]["lr"]
         for s in self.schedulers:
-            s.step()
+            if self.opt.lr_policy == "plateau":
+                s.step(self.metric)
+            else:
+                s.step()
         lr = self.optimizers[0].param_groups[0]["lr"]
         print("learning rate %.7f -> %.7f" % (old_lr, lr))
 
@@ -208,7 +211,8 @@ class Pix2PixModel(BaseModel):
         bucket.allreduce_mean_([p.grad for p in params if p.grad is not None], self.world_size, dist.all_reduce)
 
     def _backward_D(self, netD, fake, real, idx):
-        """reference backward_D_k (:267-314): 0.5 * (BCE(D(fake.detach()), 0) + BCE(D(real), 1)), gradients into netD."""
+        """reference backward_D_k (:267-314): 0.5 * (L(D(fake.detach()), False) + L(D(real), True)) with L = criterionGAN (any
+        gan_mode), gradients into netD."""
         tape = T.Tape()
         pf = netD.run(fake, tape)
         loss_fake = self.criterionGAN(pf.data, False)

@@ -402,15 +402,20 @@ def l1_mean(a, b):
     return reduce_scalar(a.contiguous(), b.contiguous(), 0, 1.0 / a.numel())
 
 
-def bce_logits_const(logits, target_is_real):
-    """GANLoss('vanilla')(logits, target_is_real) = BCEWithLogitsLoss vs a constant target (networks.py:237,:270-272)."""
-    return reduce_scalar(logits.contiguous(), None, 1, 1.0 / logits.numel(), 1.0 if target_is_real else 0.0)
+# GANLoss objectives (reference networks.py:212-278) -> (hv_reduce_scalar kind, hv_loss_grad kind)
+GAN_KINDS = {"vanilla": (1, 1), "lsgan": (5, 2), "wgangp": (3, 3)}
 
 
-def bce_logits_const_grad(logits, target_is_real, g):
-    """d(g * BCE mean)/d logits."""
+def gan_loss(logits, mode, t, sign=1.0):
+    """sign * mean over the logits of BCE-with-logits vs the constant t ('vanilla'), (x - t)^2 ('lsgan') or x ('wgangp', t unused),
+    as a device scalar."""
+    return reduce_scalar(logits.contiguous(), None, GAN_KINDS[mode][0], sign / logits.numel(), t)
+
+
+def gan_loss_grad(logits, mode, t, g, sign=1.0):
+    """d(g * gan_loss(logits, mode, t, sign))/d logits."""
     da = torch.empty_like(logits)
-    check(_L().hv_loss_grad(ptr(logits), None, 1.0 if target_is_real else 0.0, 1, float(g) / logits.numel(), None, 0, ptr(da), 0,
+    check(_L().hv_loss_grad(ptr(logits), None, float(t), GAN_KINDS[mode][1], float(g) * sign / logits.numel(), None, 0, ptr(da), 0,
                             logits.numel(), _lib.stream()))
     return da
 
@@ -475,14 +480,14 @@ class TensorTable:
         return self.dev, len(rows), self.chunks
 
 
-class FusedAdam:
+class FusedAdam(torch.optim.Optimizer):
     """torch.optim.Adam(lr, betas) semantics (pix2pix_model.py:127-130); state keys mirror torch's.  ONE kernel launch per step for
-    all parameters of the optimiser (hv_adam_step_multi); parameters with different step counts take one launch per tensor."""
+    all parameters of the optimiser (hv_adam_step_multi); parameters with different step counts take one launch per tensor.  A
+    torch.optim.Optimizer, so that torch's learning-rate schedulers drive param_groups[0]["lr"] (networks.get_scheduler)."""
 
     def __init__(self, params, lr=2e-4, betas=(0.5, 0.999), eps=1e-8):
-        self.params = [p for p in params]
-        self.param_groups = [{"params": self.params, "lr": lr, "initial_lr": lr, "betas": betas, "eps": eps}]
-        self.state = {}
+        super().__init__(params, dict(lr=lr, betas=betas, eps=eps))
+        self.params = self.param_groups[0]["params"]
         self._table = TensorTable()
         self._step = 0
 

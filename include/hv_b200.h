@@ -293,11 +293,15 @@ int hv_act_fwd(const float* x, float* y, int act, size_t count, hv_stream_t stre
 
 /* ---- A6: scalar losses.  out[0] = scale * reduce; kind 0: sum|a-b| (nn.L1Loss), 1: BCE-with-logits
  * against the constant target t (GANLoss vanilla, models/networks.py:237,:270-272), 2: count_nonzero(a)
- * (pix2pix_model.py:336), 3: sum a, 4: sum a*b.  scratch: 1024 floats.  Deterministic.     */
+ * (pix2pix_model.py:336), 3: sum a (GANLoss wgangp with scale -+1/count), 4: sum a*b, 5: sum (a-t)^2
+ * against the constant t (GANLoss lsgan).  scratch: 1024 floats.  Deterministic.  A kind outside 0..5
+ * returns HV_ERR_INVALID.                                                                    */
 int hv_reduce_scalar(const float* a, const float* b, float t, int kind, size_t count, float scale, float* out,
                      float* scratch, hv_stream_t stream);
-/* gradients: kind 0: da = g * S * sign(a-b); kind 1: da = g * S * (sigmoid(a) - t); S = 1, *scale or 1 / *scale
- * (device scalar, e.g. count_nonzero(mask)); accumulate != 0 adds into da                  */
+/* gradients: kind 0: da = g * S * sign(a-b); kind 1: da = g * S * (sigmoid(a) - t); kind 2: da = g * S * 2(a - t)
+ * (lsgan); kind 3: da = g * S (wgangp: the sign goes into g; a is not read).  S = 1, *scale or 1 / *scale
+ * (device scalar, e.g. count_nonzero(mask)); accumulate != 0 adds into da.  A kind outside 0..3 returns
+ * HV_ERR_INVALID.                                                                            */
 int hv_loss_grad(const float* a, const float* b, float t, int kind, float g, const float* scale,
                  int scale_is_reciprocal, float* da, int accumulate, size_t count, hv_stream_t stream);
 /* diceCoeff(activation='none') (pix2pix_model.py:13-39): dice_n [n], sums [n,3] kept for the backward;
