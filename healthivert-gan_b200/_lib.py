@@ -98,6 +98,9 @@ SIGNATURES = {
     "hv_dconv_workspace_bytes": (c_size_t, [c_int] * 6),
     "hv_dconv_fwd_bf16": (c_int, [c_void_p, c_void_p, c_void_p] + [c_int] * 6 + [c_void_p, c_void_p]),
     "hv_dconv_bwd_bf16": (c_int, [c_void_p] * 5 + [c_int] * 6 + [c_void_p, c_void_p]),
+    "hv_pixel_d_workspace_bytes": (c_size_t, [c_int] * 3),
+    "hv_pixel_d_fwd_bf16": (c_int, [c_void_p] * 14 + [c_int] * 6 + [c_float] * 3 + [c_void_p, c_void_p]),
+    "hv_pixel_d_bwd_bf16": (c_int, [c_void_p] * 21 + [c_int] * 6 + [c_float, c_void_p, c_void_p]),
     "hv_vol_to_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, ctypes.c_double, c_void_p]),
     "hv_slice_id_counts": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "hv_slice_prepare": (c_int, [c_void_p] * 5 + [c_int, c_int, c_int, c_int] + [c_void_p] * 10 + [c_void_p]),

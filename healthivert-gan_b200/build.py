@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libhv_b200.so")
 SOURCES = ["hv_api.cu", "sn_prepare.cu", "conv_fp32.cu", "ctx_attn.cu", "mask_ops.cu", "generator_plan.cu",
-           "conv_tc.cu", "conv_tc_api.cu", "gemm_tc.cu", "ctx_attn_tc.cu", "train_ops.cu", "slice_prep.cu", "resample.cu", "pipeline.cu", "tail_tc.cu", "stem_tc.cu", "dconv_tc.cu", "gconv_tc.cu", "inorm.cu"]
+           "conv_tc.cu", "conv_tc_api.cu", "gemm_tc.cu", "ctx_attn_tc.cu", "train_ops.cu", "slice_prep.cu", "resample.cu", "pipeline.cu", "tail_tc.cu", "stem_tc.cu", "dconv_tc.cu", "gconv_tc.cu", "inorm.cu", "pixel_d_tc.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
 

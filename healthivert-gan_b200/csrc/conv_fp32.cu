@@ -330,6 +330,7 @@ int conv2d_fwd_fp32_sub(const hv_conv_desc* d, const float* w, const float* bias
   }
   const int key = d->k * 10 + d->stride;
   switch (key) {
+    case 11: return launch_ks<1, 1>(a, st);   // PixelDiscriminator (models/networks.py:604-753) and its data gradients
     case 21: return launch_ks<2, 1>(a, st);
     case 31: return launch_ks<3, 1>(a, st);
     case 32: return launch_ks<3, 2>(a, st);

@@ -1,5 +1,5 @@
 """Drop-in mirror of the hot-path parts of the reference's ``models/networks.py`` on hand-written kernels:
-``NLayerDiscriminator`` (:555-602), ``GANLoss`` (:212-278: 'vanilla', 'lsgan', 'wgangp' without a gradient penalty),
+``NLayerDiscriminator`` (:555-602), ``PixelDiscriminator`` (in :604-753), ``GANLoss`` (:212-278: 'vanilla', 'lsgan', 'wgangp' without a gradient penalty),
 ``define_D`` (:163-206), ``get_norm_layer`` (:30-47: 'batch', 'instance', 'none'), ``Identity`` (:25-27),
 ``init_weights`` / ``init_net`` (:68-117), ``get_scheduler`` (:39-65: 'linear', 'step', 'plateau', 'cosine', torch's own
 schedulers on ``train_ops.FusedAdam``).
@@ -7,7 +7,9 @@ schedulers on ``train_ops.FusedAdam``).
 The torch ``nn.Conv2d`` / ``nn.BatchNorm2d`` objects are parameter CONTAINERS only (identical ``state_dict`` keys and identical
 initialisation streams); all arithmetic runs in libhv_b200.so.  Discriminator layouts by norm:
 'batch' ``model.{0,2,3,5,6,8,9,11}.*``; 'instance' ``model.{0,2,5,8,11}.{weight,bias}`` (InstanceNorm2d(affine=False) has no
-state, the convs before it have a bias); 'none' ``model.{0,11}.{weight,bias}`` + ``model.{2,5,8}.weight``.
+state, the convs before it have a bias); 'none' ``model.{0,11}.{weight,bias}`` + ``model.{2,5,8}.weight``.  PixelDiscriminator:
+'batch' ``net.{0,2,3,5}.*`` (no bias on convs 2 and 5); 'instance' ``net.{0,2,5}.{weight,bias}``; 'none' ``net.0.{weight,bias}`` +
+``net.{2,5}.weight``.
 """
 import functools
 
@@ -37,6 +39,66 @@ def get_norm_layer(norm_type="batch"):
     raise NotImplementedError("normalization layer [%s] is not found" % norm_type)
 
 
+def _use_bias(norm_layer):
+    if type(norm_layer) == functools.partial:
+        return norm_layer.func == nn.InstanceNorm2d
+    return norm_layer == nn.InstanceNorm2d
+
+
+def run_blocks(net, seq, x, tape=None, param_grads=True):
+    """The layer path of both discriminators: walk ``seq`` as the reference's blocks conv [-> BatchNorm2d | InstanceNorm2d | Identity]
+    [-> LeakyReLU(0.2)] on the hand-written kernels (SIMT convs, or T.conv2d_tc for the normalised 4x4 convs when net.precision is
+    'bf16').  x: tensor or tape Var; returns a Var."""
+    name = type(net).__name__
+    if not isinstance(x, T.Var):
+        x = T.Var(x.to(torch.float32).contiguous(), requires_grad=False)
+    if not x.data.is_cuda:
+        raise _lib.HvError("hv_b200 %s needs CUDA tensors (no CPU fallback)" % name)
+    mods = list(seq)
+    i = 0
+    while i < len(mods):
+        m = mods[i]
+        if not isinstance(m, nn.Conv2d):
+            raise NotImplementedError("unexpected module in the %s sequence: %r" % (name, m))
+        j = i + 1
+        norm = mods[j] if j < len(mods) and isinstance(mods[j], (nn.BatchNorm2d, nn.InstanceNorm2d, Identity)) else None
+        j += norm is not None
+        lrelu = j < len(mods) and isinstance(mods[j], nn.LeakyReLU)
+        if isinstance(norm, nn.InstanceNorm2d) and (norm.affine or norm.track_running_stats or not lrelu):
+            raise NotImplementedError("hv_b200 %s: InstanceNorm2d is built as get_norm_layer('instance') makes it" % name)
+        inorm = isinstance(norm, nn.InstanceNorm2d)
+        bare_lrelu = lrelu and not isinstance(norm, (nn.BatchNorm2d, nn.InstanceNorm2d))   # conv [-> Identity] -> LeakyReLU
+        w = m.weight.detach()
+        b = m.bias.detach() if m.bias is not None else None
+
+        def on_grad(dw, db, m=m):
+            T.accumulate_param(m.weight, dw)
+            if db is not None and m.bias is not None:
+                T.accumulate_param(m.bias, db)
+
+        h, wd = x.data.shape[2], x.data.shape[3]
+        # the tensor cores take the normalised or norm-free 4x4 convs (64->128, 128->256, 256->512: 97 % of the PatchGAN's FLOPs); a
+        # bias before InstanceNorm goes into the norm kernel
+        tc = (net.precision == "bf16" and norm is not None and (b is None or inorm) and m.kernel_size == (4, 4)
+              and m.padding == (1, 1) and m.dilation == (1, 1) and m.stride[0] in (1, 2) and m.in_channels % 8 == 0
+              and m.out_channels % 128 == 0)
+        if tc:
+            x = T.conv2d_tc(tape, x, w.contiguous(), m.stride[0], on_grad, param_grads)
+            if bare_lrelu:
+                x = T.lrelu(tape, x)
+        else:
+            x = T.conv2d(tape, [(x, HV_SRC_DIRECT)], w, b, m.kernel_size[0], m.stride[0], m.padding[0], m.dilation[0],
+                         "lrelu" if bare_lrelu else "none", (h, wd), on_grad, param_grads)
+        if isinstance(norm, nn.BatchNorm2d):
+            if not net.training:
+                raise NotImplementedError("hv_b200 %s: eval-mode BatchNorm is not on the training path" % name)
+            x = T.bn_lrelu(tape, x, norm, 0.2, param_grads)
+        elif inorm:
+            x = T.in_lrelu(tape, x, m.bias if tc else None, 0.2, norm.eps, param_grads)
+        i = j + 1 if lrelu else j
+    return x
+
+
 class NLayerDiscriminator(nn.Module):
     """PatchGAN discriminator (reference models/networks.py:555-602): conv4x4 s2 + LReLU, (conv4x4 s2 + norm + LReLU) x2,
     conv4x4 s1 + norm + LReLU, conv4x4 s1 -> 1-channel logits.  norm: BatchNorm2d (train mode only), InstanceNorm2d(affine=False)
@@ -44,10 +106,7 @@ class NLayerDiscriminator(nn.Module):
 
     def __init__(self, input_nc, ndf=64, n_layers=3, norm_layer=nn.BatchNorm2d):
         super().__init__()
-        if type(norm_layer) == functools.partial:
-            use_bias = norm_layer.func == nn.InstanceNorm2d
-        else:
-            use_bias = norm_layer == nn.InstanceNorm2d
+        use_bias = _use_bias(norm_layer)
         kw, padw = 4, 1
         sequence = [nn.Conv2d(input_nc, ndf, kernel_size=kw, stride=2, padding=padw), nn.LeakyReLU(0.2, True)]
         nf_mult = 1
@@ -67,54 +126,39 @@ class NLayerDiscriminator(nn.Module):
 
     def run(self, x, tape=None, param_grads=True):
         """Forward through the hand-written kernels.  x: tensor or tape Var; returns a Var (logits [N,1,30,30])."""
-        if not isinstance(x, T.Var):
-            x = T.Var(x.to(torch.float32).contiguous(), requires_grad=False)
-        if not x.data.is_cuda:
-            raise _lib.HvError("hv_b200 NLayerDiscriminator needs CUDA tensors (no CPU fallback)")
-        mods = list(self.model)
-        i = 0
-        while i < len(mods):
-            m = mods[i]
-            if not isinstance(m, nn.Conv2d):
-                raise NotImplementedError("unexpected module in the PatchGAN sequence: %r" % (m,))
-            # the reference's blocks: conv [-> BatchNorm2d | InstanceNorm2d | Identity] [-> LeakyReLU(0.2)]
-            j = i + 1
-            norm = mods[j] if j < len(mods) and isinstance(mods[j], (nn.BatchNorm2d, nn.InstanceNorm2d, Identity)) else None
-            j += norm is not None
-            lrelu = j < len(mods) and isinstance(mods[j], nn.LeakyReLU)
-            if isinstance(norm, nn.InstanceNorm2d) and (norm.affine or norm.track_running_stats or not lrelu):
-                raise NotImplementedError("hv_b200 NLayerDiscriminator: InstanceNorm2d is built as get_norm_layer('instance') makes it")
-            inorm = isinstance(norm, nn.InstanceNorm2d)
-            bare_lrelu = lrelu and not isinstance(norm, (nn.BatchNorm2d, nn.InstanceNorm2d))   # conv [-> Identity] -> LeakyReLU
-            w = m.weight.detach()
-            b = m.bias.detach() if m.bias is not None else None
+        return run_blocks(self, self.model, x, tape, param_grads)
 
-            def on_grad(dw, db, m=m):
-                T.accumulate_param(m.weight, dw)
-                if db is not None and m.bias is not None:
-                    T.accumulate_param(m.bias, db)
+    def forward(self, input):
+        return self.run(input).data
 
-            h, wd = x.data.shape[2], x.data.shape[3]
-            # the tensor cores take the normalised or norm-free 4x4 convs (64->128, 128->256, 256->512: 97 % of the FLOPs); a bias
-            # before InstanceNorm goes into the norm kernel
-            tc = (self.precision == "bf16" and norm is not None and (b is None or inorm) and m.kernel_size == (4, 4)
-                  and m.padding == (1, 1) and m.dilation == (1, 1) and m.stride[0] in (1, 2) and m.in_channels % 8 == 0
-                  and m.out_channels % 128 == 0)
-            if tc:
-                x = T.conv2d_tc(tape, x, w.contiguous(), m.stride[0], on_grad, param_grads)
-                if bare_lrelu:
-                    x = T.lrelu(tape, x)
-            else:
-                x = T.conv2d(tape, [(x, HV_SRC_DIRECT)], w, b, m.kernel_size[0], m.stride[0], m.padding[0], m.dilation[0],
-                             "lrelu" if bare_lrelu else "none", (h, wd), on_grad, param_grads)
-            if isinstance(norm, nn.BatchNorm2d):
-                if not self.training:
-                    raise NotImplementedError("hv_b200 NLayerDiscriminator: eval-mode BatchNorm is not on the training path")
-                x = T.bn_lrelu(tape, x, norm, 0.2, param_grads)
-            elif inorm:
-                x = T.in_lrelu(tape, x, m.bias if tc else None, 0.2, norm.eps, param_grads)
-            i = j + 1 if lrelu else j
-        return x
+
+class PixelDiscriminator(nn.Module):
+    """1x1 PatchGAN (pixelGAN) discriminator (reference models/networks.py:604-753): conv1x1 input_nc->ndf + LReLU, conv1x1
+    ndf->2ndf + norm + LReLU, conv1x1 2ndf->1 logits [N,1,H,W].
+
+    'fp32': the layer path (run_blocks).  'bf16': at ndf = 64 and input_nc = 1 the whole net is one fused computation
+    (train_ops.pixel_d: the 64->128 product on the tensor cores with bf16 operands, the 64- and 128-channel maps never leave the
+    chip); other geometries take the layer path."""
+
+    def __init__(self, input_nc, ndf=64, norm_layer=nn.BatchNorm2d):
+        super().__init__()
+        use_bias = _use_bias(norm_layer)
+        self.net = nn.Sequential(
+            nn.Conv2d(input_nc, ndf, kernel_size=1, stride=1, padding=0), nn.LeakyReLU(0.2, True),
+            nn.Conv2d(ndf, ndf * 2, kernel_size=1, stride=1, padding=0, bias=use_bias), norm_layer(ndf * 2), nn.LeakyReLU(0.2, True),
+            nn.Conv2d(ndf * 2, 1, kernel_size=1, stride=1, padding=0, bias=use_bias))
+        self.precision = "fp32"
+
+    def run(self, x, tape=None, param_grads=True):
+        """Forward through the hand-written kernels.  x: tensor or tape Var; returns a Var (logits [N,1,H,W])."""
+        norm = self.net[3]
+        if isinstance(norm, nn.InstanceNorm2d) and (norm.affine or norm.track_running_stats):
+            raise NotImplementedError("hv_b200 PixelDiscriminator: InstanceNorm2d is built as get_norm_layer('instance') makes it")
+        if self.precision == "bf16" and T.pixel_d_supported(self):
+            if isinstance(norm, nn.BatchNorm2d) and not self.training:
+                raise NotImplementedError("hv_b200 PixelDiscriminator: eval-mode BatchNorm is not on the training path")
+            return T.pixel_d(tape, x, self, param_grads)
+        return run_blocks(self, self.net, x, tape, param_grads)
 
     def forward(self, input):
         return self.run(input).data
@@ -185,12 +229,14 @@ def init_net(net, init_type="normal", init_gain=0.02, gpu_ids=[]):
 
 
 def define_D(input_nc, ndf, netD, n_layers_D=3, norm="batch", init_type="normal", init_gain=0.02, gpu_ids=[]):
-    """reference models/networks.py:163-206 ('basic' and 'n_layers' are the PatchGAN variants)."""
+    """reference models/networks.py:163-206 ('basic' and 'n_layers' are the PatchGAN variants, 'pixel' the 1x1 PixelDiscriminator)."""
     norm_layer = get_norm_layer(norm_type=norm)
     if netD == "basic":
         net = NLayerDiscriminator(input_nc, ndf, n_layers=3, norm_layer=norm_layer)
     elif netD == "n_layers":
         net = NLayerDiscriminator(input_nc, ndf, n_layers_D, norm_layer=norm_layer)
+    elif netD == "pixel":
+        net = PixelDiscriminator(input_nc, ndf, norm_layer=norm_layer)
     else:
         raise NotImplementedError("Discriminator model name [%s] is not recognized" % netD)
     return init_net(net, init_type, init_gain, gpu_ids)

@@ -358,6 +358,78 @@ def in_lrelu(tape, x, bias=None, slope=0.2, eps=1e-5, param_grads=True):
     return out
 
 
+PIXEL_D_NORM = {"Identity": 0, "BatchNorm2d": 1, "InstanceNorm2d": 2}
+
+
+def pixel_d_supported(net):
+    """True when PixelDiscriminator ``net`` has the geometry the fused kernels are built for (ndf = 64, input_nc = 1)."""
+    c1, c2 = net.net[0], net.net[2]
+    return c1.in_channels == 1 and c1.out_channels == 64 and c2.out_channels == 128
+
+
+def pixel_d(tape, x, net, param_grads=True):
+    """The whole PixelDiscriminator ``net`` (models/networks.py:604-753) as ONE tape op on the fused tensor-core kernels
+    (hv_pixel_d_fwd_bf16 / _bwd_bf16): logits [n,1,h,w].  The forward keeps only x and the norm statistics; the backward recomputes the
+    64- and 128-channel maps on chip.  BatchNorm running statistics and num_batches_tracked are updated on every call."""
+    if not isinstance(x, Var):
+        x = Var(x.to(torch.float32).contiguous(), requires_grad=False)
+    xd = x.data.contiguous()
+    if not xd.is_cuda:
+        raise _lib.HvError("hv_b200 PixelDiscriminator needs CUDA tensors (no CPU fallback)")
+    n, _, h, w = xd.shape
+    c1, norm_mod, c2, c3 = net.net[0], net.net[3], net.net[2], net.net[5]
+    kind = PIXEL_D_NORM[type(norm_mod).__name__]
+    dev = xd.device
+    L = _L()
+    d = lambda t: t.detach().contiguous() if t is not None else None
+    w1, b1, w2, b2, w3, b3 = d(c1.weight), d(c1.bias), d(c2.weight), d(c2.bias), d(c3.weight), d(c3.bias)
+    bn = norm_mod if kind == 1 else None
+    gamma, beta = (d(bn.weight), d(bn.bias)) if bn is not None else (None, None)
+    ws = torch.empty(L.hv_pixel_d_workspace_bytes(n, h, w), device=dev, dtype=torch.uint8)
+    y = torch.empty(n, 1, h, w, device=dev, dtype=torch.float32)
+    nstat = 128 * (n if kind == 2 else 1)
+    mean = torch.empty(nstat, device=dev, dtype=torch.float32) if kind else None
+    invstd = torch.empty(nstat, device=dev, dtype=torch.float32) if kind else None
+    eps = float(norm_mod.eps) if kind else 1e-5
+    check(L.hv_pixel_d_fwd_bf16(ptr(xd), ptr(w1), ptr(b1), ptr(w2), ptr(b2), ptr(gamma), ptr(beta), ptr(w3), ptr(b3),
+                                ptr(bn.running_mean) if bn is not None else None, ptr(bn.running_var) if bn is not None else None,
+                                ptr(y), ptr(mean), ptr(invstd), n, 1, 64, h, w, kind, float(bn.momentum) if bn is not None else 0.0,
+                                eps, 0.2, ptr(ws), _lib.stream()))
+    if bn is not None:
+        bn.num_batches_tracked += 1
+    out = Var(y)
+    if tape is None:
+        return out
+
+    def bwd():
+        if out.grad is None:
+            return
+        need_dx = x.requires_grad
+        if not (need_dx or param_grads):
+            return
+        e = lambda t: torch.empty_like(t) if (param_grads and t is not None) else None
+        dx = torch.empty_like(xd) if need_dx else None
+        dw1, db1, dw2, db2, dw3, db3 = e(w1), e(b1), e(w2), e(b2), e(w3), e(b3)
+        dg, dbt = e(gamma), e(beta)
+        check(L.hv_pixel_d_bwd_bf16(ptr(xd), ptr(w1), ptr(b1), ptr(w2), ptr(b2), ptr(gamma), ptr(beta), ptr(w3), ptr(b3), ptr(mean),
+                                    ptr(invstd), ptr(out.grad.contiguous()), ptr(dx), ptr(dw1), ptr(db1), ptr(dw2), ptr(db2), ptr(dg),
+                                    ptr(dbt), ptr(dw3), ptr(db3), n, 1, 64, h, w, kind, 0.2, ptr(ws), _lib.stream()))
+        if param_grads:
+            for mod, dw, db in ((c1, dw1, db1), (c2, dw2, db2), (c3, dw3, db3)):
+                accumulate_param(mod.weight, dw)
+                if db is not None:
+                    accumulate_param(mod.bias, db)
+            if bn is not None:
+                accumulate_param(bn.weight, dg)
+                accumulate_param(bn.bias, dbt)
+        if need_dx:
+            accumulate(x, dx)
+
+    tape.keep.append(ws)
+    tape.record(bwd)
+    return out
+
+
 def lrelu(tape, x):
     """LeakyReLU(0.2) as its own pass (after a tensor-core convolution, which has no activation epilogue)."""
     y = torch.empty_like(x.data)

@@ -340,6 +340,26 @@ int hv_dconv_fwd_bf16(const float* x, const float* w, float* y, int n, int cin, 
 int hv_dconv_bwd_bf16(const float* x, const float* w, const float* dy, float* dx, float* dw, int n, int cin, int cout, int h,
                       int wd, int stride, void* workspace, hv_stream_t stream);
 
+/* ---- PixelDiscriminator (netD='pixel', models/networks.py:604-753) fused on the tensor cores, ndf = 64 and input_nc = 1: conv1x1 1->64
+ * + LeakyReLU, conv1x1 64->128 + norm + LeakyReLU, conv1x1 128->1, with the 64- and 128-channel maps kept on chip.  The 64->128 product
+ * runs on tcgen05 with bf16 operands (h1, W2; dh2, W2, h1 in the backward) and fp32 accumulation; everything else is fp32.
+ * norm: 0 none, 1 batch (train-mode statistics; running_mean / running_var, both or neither, updated with momentum and the unbiased
+ * variance), 2 instance (affine-free).  x / y / dy / dx [n,1,h,w]; w1 [64], b1 [64], w2 [128,64], w3 [128] fp32; b2 [128] and b3 [1]
+ * may be NULL (no bias); gamma / beta [128] for batch norm.  save_mean / save_invstd: [128] (batch) or [n*128] (instance) written by
+ * the forward, read by the backward.  bwd: dx may be NULL; dw1 == NULL skips every parameter gradient, otherwise db1, dw2, dw3 are
+ * required and db2 / db3 / dgamma / dbeta are written where non-NULL.  workspace: hv_pixel_d_workspace_bytes(n, h, w) bytes (0 = bad
+ * extent).  No float atomics: repeated calls give the same bits.  Other ndf / input_nc: HV_ERR_INVALID before any launch.         */
+size_t hv_pixel_d_workspace_bytes(int n, int h, int w);
+int hv_pixel_d_fwd_bf16(const float* x, const float* w1, const float* b1, const float* w2, const float* b2, const float* gamma,
+                        const float* beta, const float* w3, const float* b3, float* running_mean, float* running_var, float* y,
+                        float* save_mean, float* save_invstd, int n, int cin, int ndf, int h, int w, int norm, float momentum,
+                        float eps, float slope, void* workspace, hv_stream_t stream);
+int hv_pixel_d_bwd_bf16(const float* x, const float* w1, const float* b1, const float* w2, const float* b2, const float* gamma,
+                        const float* beta, const float* w3, const float* b3, const float* save_mean, const float* save_invstd,
+                        const float* dy, float* dx, float* dw1, float* db1, float* dw2, float* db2, float* dgamma, float* dbeta,
+                        float* dw3, float* db3, int n, int cin, int ndf, int h, int w, int norm, float slope, void* workspace,
+                        hv_stream_t stream);
+
 /* ---- A8: torch.optim.Adam step (pix2pix_model.py:127-130), fused, in place */
 int hv_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, size_t count, float lr,
                  float beta1, float beta2, float eps, int step, hv_stream_t stream);

@@ -1,5 +1,6 @@
 """Config-4 measurement: pix2pix training step, batch 16 (2 samples per rank under torchrun), fp32 kernels.
 usage: python tools/bench_train.py [--batch 16] [--steps 5] [--norm batch|instance|none] [--gan-mode vanilla|lsgan|wgangp]
+                                   [--netD basic|n_layers|pixel] [--n-layers-d 3]
        |   torchrun --nproc-per-node N tools/bench_train.py"""
 import argparse
 import json
@@ -40,18 +41,22 @@ def main():
     ap.add_argument("--norm", default="batch", choices=["batch", "instance", "none"], help="the discriminators' normalisation (opt.norm)")
     ap.add_argument("--g-forward", default=None, choices=["fp32", "bf16"], help="override for the generator's conv forward alone")
     ap.add_argument("--gan-mode", default="vanilla", choices=["vanilla", "lsgan", "wgangp"], help="the GAN objective (opt.gan_mode)")
+    ap.add_argument("--netD", default="basic", choices=["basic", "n_layers", "pixel"], help="the discriminator (opt.netD)")
+    ap.add_argument("--n-layers-d", type=int, default=3, help="PatchGAN depth of --netD n_layers (opt.n_layers_D)")
     args = ap.parse_args()
     rank, world, local = sharding.world_from_env()
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    opt = synth.train_options(gpu_ids=[local], precision=args.precision, norm=args.norm, gan_mode=args.gan_mode, **({'d_precision': args.d_precision} if args.d_precision else {}),
+    opt = synth.train_options(gpu_ids=[local], precision=args.precision, norm=args.norm, gan_mode=args.gan_mode, netD=args.netD,
+                              n_layers_D=args.n_layers_d, **({'d_precision': args.d_precision} if args.d_precision else {}),
                               **({'g_forward_precision': args.g_forward} if args.g_forward else {}))
     m = Pix2PixModel(opt)
     m.setup(opt)
     m.netG.load_state_dict(synth.synthetic_generator_state_dict())
-    for k, net in enumerate((m.netD_1, m.netD_2, m.netD_3), start=1):
-        net.load_state_dict(discriminator_state_dict(k, args.norm))
+    if args.netD == "basic":       # the other discriminators keep define_D's seeded initialisation
+        for k, net in enumerate((m.netD_1, m.netD_2, m.netD_3), start=1):
+            net.load_state_dict(discriminator_state_dict(k, args.norm))
     m.train()
     m.world_size = world
     full = synth.synthetic_train_batch(n=args.batch, seed=7)
@@ -85,7 +90,7 @@ def main():
         print(json.dumps({"workload": "pix2pix optimize_parameters (BASELINE.json configs[3])", "global_batch": args.batch, "n_gpus": world,
                           "ms_per_step_device": ms, "ms_per_step_wall": wall, "ms_per_step_host_enqueue": host, "samples_per_s": args.batch / ms * 1e3,
                           "launches_per_step": (_lib.launch_count() - l0) / args.steps, "precision": args.precision, "d_precision": args.d_precision or args.precision, "norm": args.norm,
-                          "gan_mode": args.gan_mode,
+                          "gan_mode": args.gan_mode, "netD": args.netD, "n_layers_D": args.n_layers_d,
                           "losses": {k: round(v, 4) for k, v in m.get_current_losses().items()}}))
     if world > 1:
         dist.destroy_process_group()
